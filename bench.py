@@ -6,7 +6,14 @@ A *step* is one full truncated product Z = X (*) Y of two dense D^n coefficient 
 (16^6 = 16.8 M coefficients, 128 MiB per tensor, 1.2655e13 algorithmic FLOP), the largest
 single-GPU point of BASELINE.json's synthetic sweep.
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload 6x16]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload 6x16] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the timed path computed in its last step, so that two builds can be compared output for
+output: DIR/z.npy holds product coefficients (float64) and DIR/z_index.npy their flat positions in Z (float64, exact).
+The positions are all of Z when it has at most DUMP_COEFFS coefficients, else a fixed splitmix64 sample, restricted to
+the rows the timed path computes (rank 0's rows at N > 1, the CPU sample's rows with --impl reference).  The DFMA
+product kernels add partial rows in HBM with RED.ADD.F64, whose order varies, so two runs agree to rounding, not bit
+for bit: compare dumps with a relative tolerance (the parity checks below use 1e-12).
 
 N > 1 (launched by torch.distributed.run, one rank per GPU): the SAME product, output rows sharded
 over the ranks with the folded-cyclic map of genfer_b200/partition.py; Y lives block-sharded and is
@@ -55,6 +62,24 @@ def synth_inputs(n: int, d: int):
     from genfer_b200.synth import SEED_X, SEED_Y, synth_uniform
     shape = (d,) * n
     return synth_uniform(shape, SEED_X), synth_uniform(shape, SEED_Y)
+
+
+DUMP_COEFFS = 1 << 21   # at most 2 Mi coefficients: values + positions = 32 MiB, a dump small enough to keep beside a run
+DUMP_SEED = 20241020
+
+
+def dump_positions(numel: int) -> np.ndarray:
+    """Flat positions in Z written by --dump-outputs: the same for every run and build with the same --workload."""
+    if numel <= DUMP_COEFFS:
+        return np.arange(numel, dtype=np.int64)
+    from genfer_b200.synth import splitmix64
+    return np.unique((splitmix64(DUMP_SEED, DUMP_COEFFS) * numel).astype(np.int64))
+
+
+def write_outputs(out_dir: str, pos: np.ndarray, z: np.ndarray) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "z.npy"), np.ascontiguousarray(z, dtype=np.float64))
+    np.save(os.path.join(out_dir, "z_index.npy"), pos.astype(np.float64))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -327,9 +352,13 @@ def run_reference(args):
     k1s, _ = cpu_sample_rows(n, d, budget_macs=args.cpu_budget_gmac * 1e9 * 0.4)
     times, macs = [], 0.0
     for i in range(args.warmup + args.steps):
-        _, macs, dt = run_cpu_sample(x, y, k1s)
+        r, macs, dt = run_cpu_sample(x, y, k1s)
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:   # r holds rows k1s of X[0] (*) Y[0], i.e. Z[0, k1, ...]: the positions below d^(n-1)
+        pos = dump_positions(d ** n)
+        pos = pos[(pos < d ** (n - 1)) & np.isin(pos // d ** (n - 2), k1s)]
+        write_outputs(args.dump_outputs, pos, r.reshape(-1)[pos])
     total = sum(times)
     value = 2.0 * macs * len(times) / total / 1e9
     sample = (f"output rows Z[0, k1, ...], k1 in {k1s[0]}..{k1s[-1]} of the {workload_name(n, d)}: "
@@ -448,14 +477,31 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_host0 = time.perf_counter()
     e0.record()
-    for i in range(K):
+    for i in range(K - 1):
         step(i)
+    z_last = step(K - 1)                  # the product at N > 1 (None at N = 1: it is in out_rows)
     e1.record()
     torch.cuda.synchronize()
     barrier()
     t_host1 = time.perf_counter()
     launches = ctx.launch_count - l0
     clocks = sampler.stop(t_host0, t_host1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        rows = pp.rows if world == 1 else z_last.local_rows()   # the rows of Z this rank holds, in the order it holds them
+        row_len = d ** (n - 1)
+        slot = np.full(d, -1, dtype=np.int64)
+        slot[rows] = np.arange(len(rows))
+        pos = dump_positions(d ** n)
+        pos = pos[slot[pos // row_len] >= 0]
+        at = slot[pos // row_len] * row_len + pos % row_len
+        if world == 1:
+            z = out_rows.view(-1)[torch.from_numpy(at).cuda()].cpu().numpy()
+        else:
+            held = np.empty(len(rows) * row_len)
+            z_last.to_host_local_ptr(held.ctypes.data)
+            z = held[at]
+        write_outputs(args.dump_outputs, pos, z)
+    del z_last
     ms_total = e0.elapsed_time(e1)
     ms_kernel = sum(a.elapsed_time(b) for a, b in kev) / K
     t = torch.tensor([ms_total, ms_kernel], dtype=torch.float64, device="cuda")
@@ -632,7 +678,10 @@ def main():
     ap.add_argument("--no-aux", action="store_true")
     ap.add_argument("--no-sweep", action="store_true", help="skip the other four points of the synthetic sweep")
     ap.add_argument("--no-sgcl", action="store_true", help="skip the end-to-end .sgcl block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's product (sampled) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
