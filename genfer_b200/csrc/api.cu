@@ -1033,6 +1033,7 @@ int gtp_ctx_set_fast_mul(gtp_ctx* c, int enabled) {
   c->use_direct = (enabled & 65536) == 0;
   c->direct_products = (enabled & 131072) == 0;
   c->direct_products_all = (enabled & 262144) != 0;
+  c->slide_runs = (enabled & 524288) == 0;
   c->stencil_v4 = (enabled & 512) == 0;
   c->slide_tile = ((enabled >> 5) & 3) == 1 ? 4 : (((enabled >> 5) & 3) == 2 ? 8 : 0);   // A/B measurements
   enabled &= 3;

@@ -230,6 +230,7 @@ struct Ctx {
   bool use_wave = true;              // device-resident N-D div / exp / log (false: host loops of product launches; A/B tests)
   bool use_slide = true;             // sliding 1x2 kernel for dense cube slabs (false: 2x2-blocked kernel everywhere)
   int slide_tile = 0;                // 0: auto; 4 / 8: force the plane-tiled sliding plan with that many planes per slab
+  bool slide_runs = true;            // whole 16^3 slabs on the run-granular sliding kernel (false: the step-table one; A/B)
   bool stencil_v4 = true;            // stencil kernel: four coefficients per thread (false: one; A/B tests, bit 512)
   bool use_stencil = true;           // small-operand stencil product kernel (false: reference-order kernel; A/B tests)
   bool fuse_mul_linear = true;       // one-pass mul_linear kernel (false: the reference's composition, for A/B tests)

@@ -246,6 +246,180 @@ __global__ void __launch_bounds__(ST, 3) k_mul_slide(const SlideP p) {
   }
 }
 
+// k_mul_slide16's step: the columns of x in ascending order, each one's 2 (16 - j) DFMAs back to back.  In this kernel
+// the order is 2 % faster than sl_step's alternating one on B200 (6 x 16: 492.5 against 502.6 ms,
+// profiles/r03_step_order_variants.txt); ptxas then flags 604 instead of 536 of the kernel's 952 DFMAs with an operand
+// .reuse.  Interleaving z0 / z1 per accumulator was slower (514 ms).
+__device__ __forceinline__ void sl16_step(double (&z0)[16], double (&z1)[16], const double (&ya)[16], const double (&yb)[16],
+                                          const double* __restrict__ xs) {
+#pragma unroll
+  for (int jq = 0; jq < 16; jq += 2) {
+    const double2 xv = *reinterpret_cast<const double2*>(xs + jq);
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+      const int j = jq + h;
+      const double xj = h ? xv.y : xv.x;
+#pragma unroll
+      for (int kk = j; kk < 16; kk++) z0[kk] = fma(xj, ya[kk - j], z0[kk]);
+#pragma unroll
+      for (int kk = j; kk < 16; kk++) z1[kk] = fma(xj, yb[kk - j], z1[kk]);
+    }
+  }
+}
+// z1 += x (*) y: the last step of a run, whose z0 partner is the zero row y[-1] (columns from both ends, as sl_step; with
+// ascending columns here ptxas allocates the kernel's registers differently and the pair loop loses .reuse flags)
+__device__ __forceinline__ void sl16_col_z1(double (&z1)[16], const double (&y)[16], const double xj, const int jj) {
+#pragma unroll
+  for (int kk = jj; kk < 16; kk++) z1[kk] = fma(xj, y[kk - jj], z1[kk]);
+}
+__device__ __forceinline__ void sl16_step_z1(double (&z1)[16], const double (&y)[16], const double* __restrict__ xs) {
+#pragma unroll
+  for (int j = 0; j < 8; j += 2) {
+    const double2 xa = *reinterpret_cast<const double2*>(xs + j);
+    const double2 xb = *reinterpret_cast<const double2*>(xs + 14 - j);
+    sl16_col_z1(z1, y, xa.x, j);
+    sl16_col_z1(z1, y, xb.y, 15 - j);
+    sl16_col_z1(z1, y, xa.y, j + 1);
+    sl16_col_z1(z1, y, xb.x, 14 - j);
+  }
+}
+
+// Whole 16^3 slabs (D1 = D2 = L = 16, one chunk, one staged pair): the schedule is a closed form of the thread index
+// instead of a step table, and every warp walks whole runs in lockstep.
+//   lane map: warp d = row fold (row pairs {d, 7-d}, s = 2d and 14-2d), quarter-warp = team, lane c1 of the quarter-warp =
+//   plane fold (output planes {c1, 15-c1}).  All 32 lanes of a warp slide over the same row pair, so their runs have the
+//   same lengths 2d+2 (phase 0) and 16-2d (phase 1); a run is the walk a = 0 .. s+1 of one (plane pair, row pair).
+//   Each lane has 17 plane pairs t = 0..16 (t <= c1: planes (t, c1-t) -> c1, else (t-c1-1, 16-t) -> 15-c1), each with one
+//   run per phase.  Team k takes t = 4k .. 4k+3 in phase 0 and back down in phase 1 (8 whole runs); the 9 step pairs of
+//   t = 16's two runs are dealt 3 per team to teams 0..2, and team 3 multiplies zero rows instead (78 steps per team,
+//   as the step table's 312 / 306).
+// Per run the thread computes its x / y row bases once; inside it the x row moves by +L and the y row by -L.  The last
+// step of a whole run pairs z0 with the zero row and runs as a z1-only body (136 DFMA).  The accumulators change their
+// output rows only between runs, so the flush test is paid once per run.
+__global__ void __launch_bounds__(ST, 3) k_mul_slide16(const SlideP p) {
+  constexpr int LT = 16;
+  extern __shared__ __align__(16) double smem[];
+  double* Xs = smem;
+  double* Ys = smem + p.x_slab_sm;
+  const double* Zr = Ys + p.y_slab_sm;   // three zero rows: the operands of team 3's padding pairs
+  const int tid = threadIdx.x;
+  const uint4 unit = p.units[blockIdx.x];
+  {
+    const int total = (int)(p.x_slab_sm + p.y_slab_sm) + 3 * LT;
+    for (int i = tid * 2; i < total; i += ST * 2) *reinterpret_cast<double2*>(smem + i) = make_double2(0.0, 0.0);
+  }
+  unsigned k[S_MAXA], lo[S_MAXA], ext[S_MAXA];
+  {
+    unsigned rem = unit.x;
+#pragma unroll
+    for (int a = S_MAXA - 1; a >= 0; --a) {
+      if (a < p.na) {
+        unsigned len = (a == 0) ? p.rows_a0 : p.ra[a];
+        unsigned idx = rem % len;
+        rem /= len;
+        k[a] = (a == 0) ? unit.w : idx;
+        unsigned l = (k[a] + 1 > p.ya[a]) ? k[a] + 1 - p.ya[a] : 0;
+        unsigned h = (k[a] + 1 < p.xa[a]) ? k[a] + 1 : p.xa[a];
+        lo[a] = l;
+        ext[a] = h > l ? h - l : 0;
+      } else {
+        k[a] = lo[a] = 0;
+        ext[a] = 1;
+      }
+    }
+  }
+  double* out_slab = p.out + (size_t)unit.x * p.z_rows * LT;
+  const int d = tid >> 5, team = (tid >> 3) & 3, c1 = tid & 7;
+
+  double z0[LT], z1[LT], ya[LT], yb[LT];
+#pragma unroll
+  for (int i = 0; i < LT; i++) z0[i] = z1[i] = ya[i] = yb[i] = 0.0;
+  unsigned cur = 0xffffffffu;   // output row (r1 * 16 + s) of z0; z1 is the row after it
+
+  for (unsigned q = unit.y; q < unit.z; q++) {
+    __syncthreads();
+    {
+      long long xo = 0, yo = 0;
+      unsigned rem = q;
+#pragma unroll
+      for (int a = S_MAXA - 1; a >= 0; --a) {
+        if (a < p.na) {
+          unsigned j = lo[a] + rem % ext[a];
+          rem /= ext[a];
+          xo += (long long)j * p.xastr[a];
+          yo += (long long)(k[a] - j) * p.yastr[a];
+        }
+      }
+      const double2* gx = reinterpret_cast<const double2*>(p.x + xo);
+      const double2* gy = reinterpret_cast<const double2*>(p.y + yo);
+      double* ys = Ys + p.y_first;
+      constexpr int n = 16 * 16 * LT / 2;
+      for (int i = tid; i < n; i += ST) {
+        const int r = i >> 3, c = i & 7, pl = r >> 4, rr = r & 15;
+        sl_cp16(Xs + pl * p.x_plane_sm + rr * LT + 2 * c, gx + i);
+        sl_cp16(ys + pl * p.y_plane_sm + rr * LT + 2 * c, gy + i);
+      }
+    }
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    __syncthreads();
+
+#pragma unroll 1
+    for (int i = 0; i < 11; i++) {
+      int t, s, a0, npairs;
+      bool pad = false;
+      if (i < 8) {   // whole runs
+        const int ph = i >> 2;
+        t = 4 * team + (ph ? 3 - (i & 3) : (i & 3));
+        s = ph ? 14 - 2 * d : 2 * d;
+        a0 = 0;
+        npairs = s / 2 + 1;
+      } else {       // step pair pr of t = 16's runs: pairs 0..d belong to the phase-0 run, d+1..8 to the phase-1 run
+        const int pr = 3 * team + (i - 8);
+        t = 16;
+        if (pr <= d) { s = 2 * d; a0 = 2 * pr; }
+        else { s = 14 - 2 * d; a0 = 2 * (pr - d - 1); }
+        pad = pr >= 9;
+        npairs = 1;
+      }
+      const int r1 = t <= c1 ? c1 : 15 - c1;
+      const int j1 = t <= c1 ? t : t - c1 - 1;
+      const double* xs = Xs + j1 * p.x_plane_sm + a0 * LT;
+      const double* ys = Ys + (r1 - j1) * p.y_plane_sm + (s - a0 + 1) * LT;   // y row s - a0 (row -1 is the zero row)
+      unsigned zrow = (unsigned)(r1 * 16 + s);
+      if (pad) { xs = Zr; ys = Zr + LT; zrow = cur; }
+      if (zrow != cur) {
+        if (cur != 0xffffffffu) {
+          double* dst = out_slab + (size_t)cur * LT;
+          sl_flush<LT>(z0, dst, true);
+          sl_flush<LT>(z1, dst + LT, true);
+        }
+        cur = zrow;
+      }
+      sl_load<LT>(yb, ys + LT);
+      const int whole = i < 8 ? npairs - 1 : npairs;
+#pragma unroll 1   // one copy of the pair body: the four warps sit in runs of different lengths
+      for (int m = 0; m < whole; m++) {
+        sl_load<LT>(ya, ys);
+        sl16_step(z0, z1, ya, yb, xs);
+        sl_load<LT>(yb, ys - LT);
+        sl16_step(z0, z1, yb, ya, xs + LT);
+        xs += 2 * LT;
+        ys -= 2 * LT;
+      }
+      if (i < 8) {   // a = s, s + 1
+        sl_load<LT>(ya, ys);
+        sl16_step(z0, z1, ya, yb, xs);
+        sl16_step_z1(z1, ya, xs + LT);
+      }
+    }
+  }
+  if (cur != 0xffffffffu) {
+    double* dst = out_slab + (size_t)cur * LT;
+    sl_flush<LT>(z0, dst, true);
+    sl_flush<LT>(z1, dst + LT, true);
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
@@ -494,6 +668,7 @@ static void build_slide_table_tiled(const SlideGeom& g, std::vector<uint2>* tabl
 struct SlidePlan {
   BufP table, units;
   unsigned n_units = 0;
+  bool runs = false;   // k_mul_slide16 (no step table)
   SlideP p;
   SlideGeom g;
 };
@@ -519,14 +694,27 @@ template <int LT> static void slide_launch_lt(Ctx& ctx, const SlidePlan& pl, con
   else GTP_LAUNCH(ctx, (k_mul_slide<LT, false>), pl.n_units, pl.g.threads, pl.g.smem, p);
 }
 
+static void slide_launch_runs(Ctx& ctx, const SlidePlan& pl, const SlideP& p) {
+  static size_t configured[64] = {};
+  if (configured[ctx.device & 63] < pl.g.smem) {
+    GTP_CUDA(cudaFuncSetAttribute(k_mul_slide16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
+    configured[ctx.device & 63] = pl.g.smem;
+  }
+  GTP_LAUNCH(ctx, k_mul_slide16, pl.n_units, pl.g.threads, pl.g.smem, p);
+}
+
 void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
   SlideGeom g;
   GTP_CHECK(slide_geom(ctx, a, &g), GTP_ERR_ARG, "sliding product kernel not applicable");
+  // whole 16^3 slabs run on k_mul_slide16 (ctx.slide_runs = false: the table-driven kernel, for A/B measurements)
+  const bool runs = ctx.slide_runs && g.nt == 1 && g.D1 == 16 && g.D2 == 16 && g.lt == 16 && g.lc == 1 && g.G == 1 && g.threads == ST;
+  if (runs) g.smem += 3 * 16 * sizeof(double);   // the zero rows of the padding pairs
   SlideKey key;
   key.v.insert(key.v.end(), a.xs.begin(), a.xs.end());
   key.v.insert(key.v.end(), a.ys.begin(), a.ys.end());
   key.v.insert(key.v.end(), a.rs.begin(), a.rs.end());
   key.v.push_back(g.T1);
+  key.v.push_back(runs ? 1 : 0);
   key.v.push_back(a.row_begin);
   key.v.push_back(a.row_step);
   key.v.push_back(a.row_count);
@@ -539,6 +727,7 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
   } else {
     pl = std::make_shared<SlidePlan>();
     pl->g = g;
+    pl->runs = runs;
     SlideP& p = pl->p;
     memset(&p, 0, sizeof(p));
     const int nd = g.nd, nr = g.na, tiled = g.nt > 1 ? 1 : 0, na = nr + tiled;
@@ -578,7 +767,8 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
     p.z_up = (unsigned)g.lc;
     p.G = g.G;
     std::vector<uint2> table;
-    if (tiled) build_slide_table_tiled(g, &table, &p.nsteps_lo, &p.nsteps);
+    if (runs) p.nsteps_lo = p.nsteps = 0;
+    else if (tiled) build_slide_table_tiled(g, &table, &p.nsteps_lo, &p.nsteps);
     else build_slide_table(g, &table, &p.nsteps_lo, &p.nsteps);
     p.nsteps += p.nsteps_lo;
     // ---- work units (as in kernels_mul_blk.cu) ----
@@ -623,7 +813,8 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
     for (size_t i = 0; i < units.size(); i++) hu[i] = make_uint4(units[i].ka, units[i].q0, units[i].q1, units[i].k0);
     pl->table = ctx.alloc(table.size() + 1);
     pl->units = ctx.alloc(hu.size() * 2 + 1);
-    GTP_CUDA(cudaMemcpyAsync(pl->table->d, table.data(), table.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx.stream));
+    if (!table.empty())
+      GTP_CUDA(cudaMemcpyAsync(pl->table->d, table.data(), table.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx.stream));
     if (!hu.empty())
       GTP_CUDA(cudaMemcpyAsync(pl->units->d, hu.data(), hu.size() * sizeof(uint4), cudaMemcpyHostToDevice, ctx.stream));
     ctx.sync();
@@ -639,7 +830,12 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
   u64 row_elems = 1;
   for (int d = 1; d < a.ndim; d++) row_elems *= a.rs[d];
   GTP_CUDA(cudaMemsetAsync(a.out, 0, a.row_count * row_elems * sizeof(double), ctx.stream));
-  if (pl->n_units == 0 || p.nsteps == 0) return;
+  if (pl->n_units == 0) return;
+  if (pl->runs) {
+    slide_launch_runs(ctx, *pl, p);
+    return;
+  }
+  if (p.nsteps == 0) return;
   switch ((int)pl->g.lt) {
     case 8: slide_launch_lt<8>(ctx, *pl, p); break;
     case 10: slide_launch_lt<10>(ctx, *pl, p); break;

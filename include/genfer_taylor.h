@@ -80,7 +80,8 @@ uint64_t gtp_ctx_launch_count(gtp_ctx* ctx);
  * +32768 plain small-operand products on the row-staged kernel too (slower than the gather kernel; A/B),
  * +65536 row-walking plain-load variant of the Horner loop (k_horner_direct, the default for tensors from 2^17 coefficients
  * with rows of at least 48) off, +131072 plain small-operand products with rows of at least 192 coefficients stay on the gather
- * kernel instead of k_horner_direct, +262144 plain small-operand products of any row length on k_horner_direct (A/B).
+ * kernel instead of k_horner_direct, +262144 plain small-operand products of any row length on k_horner_direct (A/B),
+ * +524288 whole 16^3 slabs on the step-table sliding kernel instead of the run-granular k_mul_slide16 (A/B).
  * Environment (read at gtp_ctx_create): GTP_DIRECT_MIN / GTP_DIRECT_CTAS tune k_horner_direct's size threshold and CTAs per SM; GTP_LAUNCH_HIST=1 prints per-kernel launch counts and host-time shares when the
  * context is destroyed; GTP_NO_SCALAR_POOL=1 / GTP_NO_FUSED_CLS=1 switch the host-written scalar slots / the fused
  * classification off. */
