@@ -1018,9 +1018,7 @@ void* gtp_ctx_stream(gtp_ctx* c) { return c ? (void*)c->stream : nullptr; }
 uint64_t gtp_ctx_launch_count(gtp_ctx* c) { return c ? c->launches : 0; }
 int gtp_ctx_set_fast_mul(gtp_ctx* c, int enabled) {
   if (!c) return GTP_ERR_ARG;
-  // bit 2 (value 4) switches the blocked kernel's structured item tables off (A/B measurements)
-  c->blk_fold_tables = (enabled & 4) == 0;
-  c->blk_octet = (enabled & 8) != 0;   // experimental
+  // bits 4 and 8 are ignored (they selected the blocked kernel's retired table variants)
   c->use_slide = (enabled & 16) == 0;
   c->fuse_mul_linear = (enabled & 128) == 0;
   c->use_stencil = (enabled & 256) == 0;

@@ -214,7 +214,7 @@ struct Ctx {
   u64 rb_seq = 0;               // sequence number of the last zero-copy read-back request
   Readback* rb_host_dev = nullptr;  // device alias of rb_host (mapped pinned memory)
   int fast_mul = 1;  // 0: reference-order kernel only, 1: auto, 2: force the blocked kernel even on tiny products (tests)
-  std::shared_ptr<void> blk_plans;   // per-context cache of product plans (kernels_mul_blk.cu)
+  std::shared_ptr<void> blk_plans;   // per-context caches of DFMA product plans (kernels_mul_blk.cu, dfma_plan_slot)
   std::shared_ptr<void> slide_plans; // same for kernels_mul_slide.cu
   std::shared_ptr<void> wave_tables; // level tables of the device-resident recurrences (kernels_wave.cu)
   bool bulk_products = false;        // also run plain small-operand products on the row-staged kernel (A/B; slower than the gather kernel)
@@ -234,8 +234,6 @@ struct Ctx {
   bool stencil_v4 = true;            // stencil kernel: four coefficients per thread (false: one; A/B tests, bit 512)
   bool use_stencil = true;           // small-operand stencil product kernel (false: reference-order kernel; A/B tests)
   bool fuse_mul_linear = true;       // one-pass mul_linear kernel (false: the reference's composition, for A/B tests)
-  bool blk_octet = false;            // experimental octet tables for single-plane slabs (8 staged pairs = 8 lanes)
-  bool blk_fold_tables = true;       // structured (folded) item tables for dense cube slabs; false: evenly dealt
 
   std::shared_ptr<ScalarPool> scalars;   // created with the context
   static constexpr unsigned CLS_RING = 1 << 16;

@@ -1,5 +1,7 @@
 // Launcher declarations for the device kernels of libgenfer_taylor (sm_100a).
 #pragma once
+#include <mutex>
+
 #include "common.hpp"
 
 namespace gtp {
@@ -17,6 +19,26 @@ constexpr int MAXD = GTP_MAX_NDIM;
     }                                                                           \
     GTP_CUDA(cudaGetLastError());                                               \
   } while (0)
+
+// Lets `fn` launch with `bytes` of dynamic shared memory on `device` (the current device): raises the kernel's limit when
+// it is below `bytes` and never lowers it.  The record is per (kernel, device) and shared by all contexts, which may live
+// on different threads.
+inline void allow_dyn_smem(const void* fn, int device, size_t bytes) {
+  static std::mutex mu;
+  static std::map<std::pair<const void*, int>, size_t> limit;
+  std::lock_guard<std::mutex> lock(mu);
+  size_t& cur = limit[{fn, device}];
+  if (cur >= bytes) return;
+  GTP_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  cur = bytes;
+}
+template <class F> void allow_dyn_smem(F* fn, int device, size_t bytes) { allow_dyn_smem((const void*)fn, device, bytes); }
+
+// 16-byte global -> shared copy that bypasses L1 (the DFMA product kernels stage their slabs with it)
+__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
+  unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
+}
 
 // ---------------------------------------------------------------------------------------------
 // Generic N-D element-wise / gather kernel.  Iterates the box `ext` (after host-side coalescing of
@@ -180,6 +202,33 @@ double args_macs(const MulArgs& a);   // MACs of the rows this launch computes
 // Products below this many MACs stay on the reference-order kernel (bit-exact, and launch-bound anyway); above it the
 // DFMA kernels run even when only a few slabs exist (their units split the j box, so a handful of slabs still fills the SMs)
 constexpr double DFMA_MIN_MACS = 1 << 20;
+
+// Host plan path of the DFMA product kernels (the 2x2-blocked k_mul_blk and the sliding k_mul_slide / k_mul_slide16).
+// Chunk length of a last axis of `l` doubles: the longest of 16, 14, 12, 10, 8 that divides it; 0: none does.
+u64 dfma_chunk(u64 l);
+// `doubles` rounded up to an even count whose half is odd: shared-memory strides of an odd number of 16-byte groups put
+// the planes / staged slabs that lockstep lanes read into different bank groups.
+inline u64 odd_groups(u64 doubles) {
+  doubles = (doubles + 1) / 2 * 2;
+  if ((doubles / 2) % 2 == 0) doubles += 2;
+  return doubles;
+}
+// Work units {packed output slab index, q0, q1, k along A axis 0}: each output slab of the A axes (extents axs / ays / ars
+// of X, Y and Z; axis 0 walks the launch's rows) splits its box of (X slab, Y slab) pairs into chunks [q0, q1) of whole
+// rounds of G pairs.  Units run at least 8 rounds unless that leaves some of the `slots` resident CTAs idle.  Sorted
+// longest first (LPT).
+std::vector<uint4> dfma_units(const MulArgs& a, const Shape& axs, const Shape& ays, const Shape& ars, int G, u64 slots);
+// Device arrays of a cached plan; the kernel-specific plans derive from it.
+struct DfmaPlan {
+  BufP table, units;   // step table (uint2 entries) and work units (uint4)
+  unsigned n_units = 0;
+};
+// The entry of `cache` (a context's plan slot) for this product's shapes and rows and the caller's `extra` word.  Empty on
+// a miss: the caller builds the plan and stores it there.  A cache that holds more than 64 plans is cleared first.
+std::shared_ptr<void>& dfma_plan_slot(std::shared_ptr<void>& cache, const MulArgs& a, u64 extra);
+// Copies the step table and the units to new device arrays of `pl` (empty arrays are not copied) and waits for the copy.
+void dfma_upload(Ctx& ctx, DfmaPlan* pl, const std::vector<uint2>& table, const std::vector<uint4>& units);
+
 void fp64_peak_probe(Ctx& ctx, int kind, int iters, double* flops, double* ms);
 
 // ---------------------------------------------------------------------------------------------

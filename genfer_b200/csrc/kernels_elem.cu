@@ -710,11 +710,7 @@ void launch_shift_down(Ctx& ctx, const double* in, double* out, u64 outer, u64 l
              (outer + SD_LANES - 1) / SD_LANES < (1u << 31)) {
     unsigned pad = (unsigned)((len & 1) ? len : len + 1);
     size_t smem = (size_t)SD_LANES * pad * sizeof(double);
-    static bool configured[64] = {};
-    if (!configured[ctx.device & 63]) {
-      GTP_CUDA(cudaFuncSetAttribute(k_shift_down_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, SD_LANES * 65 * 8));
-      configured[ctx.device & 63] = true;
-    }
+    allow_dyn_smem(k_shift_down_tile, ctx.device, SD_LANES * 65 * 8);
     unsigned grid = (unsigned)((outer + SD_LANES - 1) / SD_LANES);
     GTP_LAUNCH(ctx, k_shift_down_tile, grid, SD_LANES, smem, in, out, outer, (unsigned)len, (unsigned)n, (unsigned)out_len, pad);
   } else {

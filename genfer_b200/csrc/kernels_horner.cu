@@ -881,17 +881,12 @@ static bool launch_rows_variant(Ctx& ctx, const HornerP& p, int add_mode, const 
   }
   if (c < 0) return false;
   const void* fn;
-  int bucket;
-  if (p.nt <= 2) { fn = (const void*)k_horner_rows<2>; bucket = 0; }
-  else if (p.nt <= 4) { fn = (const void*)k_horner_rows<4>; bucket = 1; }
-  else if (p.nt <= 8) { fn = (const void*)k_horner_rows<8>; bucket = 2; }
-  else if (p.nt <= 16) { fn = (const void*)k_horner_rows<16>; bucket = 3; }
-  else { fn = (const void*)k_horner_rows<32>; bucket = 4; }
-  static size_t configured[5][64] = {};
-  if (configured[bucket][ctx.device & 63] < smem) {
-    GTP_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured[bucket][ctx.device & 63] = smem;
-  }
+  if (p.nt <= 2) fn = (const void*)k_horner_rows<2>;
+  else if (p.nt <= 4) fn = (const void*)k_horner_rows<4>;
+  else if (p.nt <= 8) fn = (const void*)k_horner_rows<8>;
+  else if (p.nt <= 16) fn = (const void*)k_horner_rows<16>;
+  else fn = (const void*)k_horner_rows<32>;
+  allow_dyn_smem(fn, ctx.device, smem);
   int per_sm = 0;
   GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, HB_T, smem));
   if (per_sm < 1) return false;

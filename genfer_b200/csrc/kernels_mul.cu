@@ -5,8 +5,8 @@
 // coefficient.  It performs the multiply and the add separately (DMUL + DADD, no FMA) and
 // in exactly the reference's nesting order -- outer axes ascending, the innermost non-unit axis
 // summed from zero and then added (mul_1d :972-982 feeding `*z += o` :998) -- so its results are
-// bit-identical to the reference f64 path.  The register-blocked DFMA kernel lives in kernels_mul_blk.cu;
-// launch_mul() picks between them.
+// bit-identical to the reference f64 path.  The DFMA kernels live in kernels_mul_blk.cu and kernels_mul_slide.cu
+// (their shared host plan path is here); launch_mul() picks between them.
 #include <algorithm>
 
 #include "kernels.cuh"
@@ -137,6 +137,84 @@ double mul_macs(const Shape& xs, const Shape& ys, const Shape& rs) {
     total *= s;
   }
   return total;
+}
+
+// ------------------------------------------------------------------------------------------
+// Host plan path shared by the DFMA kernels (kernels_mul_blk.cu, kernels_mul_slide.cu)
+// ------------------------------------------------------------------------------------------
+u64 dfma_chunk(u64 l) {
+  for (u64 lt : {16, 14, 12, 10, 8})
+    if (l % lt == 0) return lt;
+  return 0;
+}
+
+std::vector<uint4> dfma_units(const MulArgs& a, const Shape& axs, const Shape& ays, const Shape& ars, int G, u64 slots) {
+  const int na = (int)axs.size();
+  u64 n_slabs = a.row_count;
+  for (int d = 1; d < na; d++) n_slabs *= ars[d];
+  auto row_of = [&](u64 idx) -> u64 { return a.rows.empty() ? a.row_begin + idx * a.row_step : a.rows[idx]; };
+  std::vector<u64> boxes(n_slabs);
+  std::vector<unsigned> k0s(n_slabs, 0);
+  u64 total_pairs = 0;
+  for (u64 s = 0; s < n_slabs; s++) {
+    u64 rem = s, box = 1;
+    for (int d = na - 1; d >= 0; --d) {
+      u64 len = (d == 0) ? a.row_count : ars[d];
+      u64 idx = rem % len;
+      rem /= len;
+      u64 k = (d == 0) ? row_of(idx) : idx;
+      if (d == 0) k0s[s] = (unsigned)k;
+      u64 lo = sat_sub(k + 1, ays[d]), hi = std::min(k + 1, axs[d]);
+      box *= hi > lo ? hi - lo : 0;
+    }
+    boxes[s] = box;
+    total_pairs += box;
+  }
+  // at least 8 rounds per unit amortise its set-up -- unless that leaves resident-CTA slots empty (mid-size products)
+  const u64 min_chunk = total_pairs >= slots * 8 * (u64)G ? 8 * (u64)G : (u64)G;
+  u64 chunk = std::max<u64>(min_chunk, total_pairs / (slots * 16) + 1);
+  chunk = (chunk + G - 1) / G * G;   // whole rounds
+  std::vector<uint4> units;
+  for (u64 s = 0; s < n_slabs; s++) {
+    u64 box = boxes[s];
+    if (!box) continue;
+    u64 parts = (box + chunk - 1) / chunk;
+    u64 per = (box + parts - 1) / parts;
+    per = (per + G - 1) / G * G;
+    for (u64 q0 = 0; q0 < box; q0 += per) units.push_back(make_uint4((unsigned)s, (unsigned)q0, (unsigned)std::min(box, q0 + per), k0s[s]));
+  }
+  std::stable_sort(units.begin(), units.end(), [](const uint4& x, const uint4& y) { return (x.z - x.y) > (y.z - y.y); });
+  return units;
+}
+
+using DfmaPlanCache = std::map<std::vector<u64>, std::shared_ptr<void>>;
+std::shared_ptr<void>& dfma_plan_slot(std::shared_ptr<void>& cache, const MulArgs& a, u64 extra) {
+  if (!cache) cache = std::make_shared<DfmaPlanCache>();
+  auto& plans = *std::static_pointer_cast<DfmaPlanCache>(cache);
+  std::vector<u64> key{(u64)a.ndim};   // fixes where the shapes end and the row list begins
+  key.insert(key.end(), a.xs.begin(), a.xs.end());
+  key.insert(key.end(), a.ys.begin(), a.ys.end());
+  key.insert(key.end(), a.rs.begin(), a.rs.end());
+  key.push_back(a.row_begin);
+  key.push_back(a.row_step);
+  key.push_back(a.row_count);
+  key.push_back(extra);
+  key.insert(key.end(), a.rows.begin(), a.rows.end());
+  auto it = plans.find(key);
+  if (it != plans.end()) return it->second;
+  if (plans.size() > 64) plans.clear();
+  return plans[key];
+}
+
+void dfma_upload(Ctx& ctx, DfmaPlan* pl, const std::vector<uint2>& table, const std::vector<uint4>& units) {
+  pl->n_units = (unsigned)units.size();
+  pl->table = ctx.alloc(table.size() + 1);   // sizes in doubles: a uint2 is one, a uint4 two
+  pl->units = ctx.alloc(units.size() * 2 + 1);
+  if (!table.empty())
+    GTP_CUDA(cudaMemcpyAsync(pl->table->d, table.data(), table.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx.stream));
+  if (!units.empty())
+    GTP_CUDA(cudaMemcpyAsync(pl->units->d, units.data(), units.size() * sizeof(uint4), cudaMemcpyHostToDevice, ctx.stream));
+  ctx.sync();   // the host arrays are the caller's temporaries
 }
 
 // implemented in kernels_mul_blk.cu / kernels_mul_slide.cu
@@ -505,8 +583,7 @@ static bool launch_mul_stencil(Ctx& ctx, const MulArgs& a) {
 // ------------------------------------------------------------------------------------------
 static u64 pad_chunkable(u64 l) {
   for (u64 c = l;; c++)
-    for (u64 lt : {16, 14, 12, 10, 8})
-      if (c % lt == 0) return c;
+    if (dfma_chunk(c)) return c;
 }
 // 0: no padded plan; 2 / 3: zero-extend and run the blocked / sliding kernel on `best`
 static int pad_plan(const Ctx& ctx, const MulArgs& a, MulArgs* out_best) {

@@ -159,11 +159,7 @@ bool launch_mul_axis(Ctx& ctx, const MulArgs& a) {
   if (inner == 1) {
     const size_t smem = (2 * Ls + AX_TB) * sizeof(double);
     if (smem > 200 * 1024 || outer > 65535) return false;
-    static size_t configured[64] = {};
-    if (configured[ctx.device & 63] < smem) {
-      GTP_CUDA(cudaFuncSetAttribute(k_mul_axis_row, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 48 * 1024)));
-      configured[ctx.device & 63] = std::max<size_t>(smem, 48 * 1024);
-    }
+    allow_dyn_smem(k_mul_axis_row, ctx.device, std::max<size_t>(smem, 48 * 1024));
     dim3 grid((unsigned)((Lr + AX_TB - 1) / AX_TB), (unsigned)outer);
     GTP_LAUNCH(ctx, k_mul_axis_row, grid, AX_TB, smem, p);
     return true;

@@ -18,13 +18,11 @@
 //   host-built table that deals them EVENLY to the threads, ordered by z row block so a thread flushes
 //   (RED.ADD.F64 to HBM) only when its block changes.
 // * A-axes: work unit = (output slab kA, chunk [q0,q1) of the jA box), longest first (LPT).
-#include <map>
-
 #include "kernels.cuh"
 
 namespace gtp {
 
-constexpr int BT = 128;       // threads per CTA (256 in octet mode when 8 slab pairs need a whole SM's shared memory)
+constexpr int BT = 128;       // threads per CTA
 constexpr int B_MAXA = 6;
 constexpr int B_MAXG = 8;
 
@@ -42,7 +40,6 @@ struct BlkP {
   unsigned x_slab_sm, y_slab_sm;                 // per staged slab
   unsigned x_pair_off, y_pair_off;               // distance between the two rows of a pair (Lc*ROW)
   int G;
-  int octet;               // 1: table has one column per 8-thread octet, lane = staged slab g (see build_octet_table)
   int nsteps_lo, nsteps;   // steps [0, nsteps_lo) hold `lo` items, [nsteps_lo, nsteps) `hi` items
   const uint2* table;    // [nsteps][BT]
   const uint4* units;    // {packed kA index, q0, q1, k along A axis 0}
@@ -56,11 +53,6 @@ struct BlkP {
 constexpr unsigned BE_VALID = 1u << 31;
 
 template <int LT> struct BRow { static constexpr int value = ((LT / 2) % 2 == 1) ? LT : LT + 2; };
-
-__device__ __forceinline__ void blk_cp16(void* smem, const void* gmem) {
-  unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
-}
 
 template <int LT>
 __device__ __forceinline__ void blk_flush(double (&z)[LT], double* __restrict__ dst, bool write) {
@@ -113,7 +105,7 @@ __device__ __forceinline__ void blk_item(double (&z0)[LT], double (&z1)[LT], dou
 }
 
 template <int LT, bool CHUNKED>
-__global__ void __launch_bounds__(256) k_mul_blk(const BlkP p) {
+__global__ void __launch_bounds__(BT) k_mul_blk(const BlkP p) {
   constexpr int ROW = BRow<LT>::value;
   constexpr int V2 = LT / 2;
   extern __shared__ __align__(16) double smem[];
@@ -122,11 +114,6 @@ __global__ void __launch_bounds__(256) k_mul_blk(const BlkP p) {
   const int tid = threadIdx.x;
   const int bt = blockDim.x;
   const uint4 unit = p.units[blockIdx.x];
-  // table column of this thread, and the staged slab its entries refer to (octet mode: lane = g)
-  const int tcols = p.octet ? (bt >> 3) : bt;
-  const int tcol = p.octet ? (tid >> 3) : tid;
-  const unsigned lane_g = p.octet ? (unsigned)(tid & 7) : 0u;
-  const unsigned lane_xoff = lane_g * p.x_slab_sm, lane_yoff = lane_g * p.y_slab_sm;
 
   // zero the whole staging area once: padding rows (odd b2) must read as zeros forever
   {
@@ -185,12 +172,12 @@ __global__ void __launch_bounds__(256) k_mul_blk(const BlkP p) {
       for (int i = tid; i < nx; i += bt) {
         int r = i / V2, c = i - r * V2;
         int pl = r / (int)p.x_prow, rr = r - pl * (int)p.x_prow;
-        blk_cp16(xs + pl * p.x_plane_sm + rr * ROW + 2 * c, gx + i);
+        cp_async16(xs + pl * p.x_plane_sm + rr * ROW + 2 * c, gx + i);
       }
       for (int i = tid; i < ny; i += bt) {
         int r = i / V2, c = i - r * V2;
         int pl = r / (int)p.y_prow, rr = r - pl * (int)p.y_prow;
-        blk_cp16(ys + pl * p.y_plane_sm + rr * ROW + 2 * c, gy + i);
+        cp_async16(ys + pl * p.y_plane_sm + rr * ROW + 2 * c, gy + i);
       }
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
@@ -208,12 +195,12 @@ __global__ void __launch_bounds__(256) k_mul_blk(const BlkP p) {
       if (cnt <= 0) continue;
       int step = fwd ? s_begin : s_end - 1;
       const int dstep = fwd ? 1 : -1;
-      uint2 e = p.table[step * tcols + tcol];
+      uint2 e = p.table[step * bt + tid];
       for (int s = 0; s < cnt; ++s) {
         step += dstep;
         uint2 en = make_uint2(0u, 0u);
-        if (s + 1 < cnt) en = p.table[step * tcols + tcol];
-        if ((e.x & BE_VALID) && (int)(((e.x >> 20) & 15u) + lane_g) < ng) {
+        if (s + 1 < cnt) en = p.table[step * bt + tid];
+        if ((e.x & BE_VALID) && (int)((e.x >> 20) & 15u) < ng) {
           const unsigned zkey = ((e.y >> 20) << 2) | ((e.x >> 25) & 3u);
           if (zkey != cur) {
             if (cur != 0xffffffffu) {
@@ -224,8 +211,8 @@ __global__ void __launch_bounds__(256) k_mul_blk(const BlkP p) {
             }
             cur = zkey;
           }
-          const double* xs = Xs + (e.x & 0xfffffu) + lane_xoff;
-          const double* ys = Ys + (e.y & 0xfffffu) + lane_yoff;
+          const double* xs = Xs + (e.x & 0xfffffu);
+          const double* ys = Ys + (e.y & 0xfffffu);
           if (hi) blk_item<LT, true>(z0, z1, z2, xs, xs + p.x_pair_off, ys, ys + p.y_pair_off);
           else blk_item<LT, false>(z0, z1, z2, xs, xs + p.x_pair_off, ys, ys + p.y_pair_off);
         }
@@ -252,26 +239,18 @@ struct BlkGeom {
   u64 row;             // padded row length in smem (doubles)
   u64 xplane, yplane, xslab, yslab;   // smem strides (doubles)
   int G;
-  int bt;              // threads per CTA
-  bool octet;          // lanes of an 8-thread octet = the 8 staged slab pairs
   size_t smem;
 };
 
 struct BlkGeom;
 static bool blk_dense(const BlkGeom& g);
 
-static u64 pick_chunk(u64 ltt) {
-  for (u64 lt : {16, 14, 12, 10, 8})
-    if (ltt % lt == 0) return lt;
-  return 0;
-}
-
-static bool blk_geom(const MulArgs& a, BlkGeom* g, bool allow_octet = false) {
+static bool blk_geom(const MulArgs& a, BlkGeom* g) {
   const int nd = a.ndim;
   if (nd < 3) return false;
   const u64 ltt = a.rs[nd - 1];
   if (a.xs[nd - 1] != ltt || a.ys[nd - 1] != ltt) return false;
-  const u64 lt = pick_chunk(ltt);
+  const u64 lt = dfma_chunk(ltt);
   if (!lt) return false;
   for (int d = 0; d < nd; d++)
     if (a.xs[d] == 0 || a.ys[d] == 0 || a.rs[d] == 0) return false;
@@ -284,13 +263,9 @@ static bool blk_geom(const MulArgs& a, BlkGeom* g, bool allow_octet = false) {
     u64 xrows = ((g->xb2 + 1) / 2 * 2) * g->lc, yrows = ((g->yb2 + 1) / 2 * 2) * g->lc;
     g->xplane = xrows * g->row + 2;   // +2 doubles: consecutive planes start in different 16-byte bank groups
     g->yplane = yrows * g->row + 2;
-    g->xslab = xb1 * g->xplane + 2;
-    g->yslab = yb1 * g->yplane + 2;
-    g->xslab = (g->xslab + 1) / 2 * 2;
-    g->yslab = (g->yslab + 1) / 2 * 2;
     // staged slabs g = 0..G-1 start in different 16-byte bank groups: slab stride = odd number of groups
-    if ((g->xslab / 2) % 2 == 0) g->xslab += 2;
-    if ((g->yslab / 2) % 2 == 0) g->yslab += 2;
+    g->xslab = odd_groups(xb1 * g->xplane + 2);
+    g->yslab = odd_groups(yb1 * g->yplane + 2);
   };
   // try the 3-axis slab first
   const size_t budget = 100 * 1024;   // two CTAs per SM
@@ -312,17 +287,6 @@ static bool blk_geom(const MulArgs& a, BlkGeom* g, bool allow_octet = false) {
   const u64 pair = (g->xslab + g->yslab) * 8;
   if (pair > budget) return false;
   g->G = (int)std::max<u64>(1, std::min<u64>(B_MAXG, budget / pair));
-  g->bt = BT;
-  g->octet = false;
-  if (g->fold_b1 && allow_octet) {
-    // (experimental, off by default: conflict-free but RED-bound, see DESIGN.md 4.1)
-    // single-plane slabs: stage 8 pairs and let the 8 lanes of an octet run the same item on the 8 pairs
-    if (8 * pair <= budget) {
-      g->G = 8; g->octet = true;
-    } else if (8 * pair <= 200 * 1024) {
-      g->G = 8; g->octet = true; g->bt = 256;   // one 256-thread CTA per SM
-    }
-  }
   if (g->G * std::max(g->xslab, g->yslab) >= (1u << 20)) return false;
   g->smem = (size_t)g->G * pair;
   return true;
@@ -342,7 +306,6 @@ struct BlkItem { unsigned xoff, yoff, zrow, kind, zv; };
 // Items of ONE slab pair, grouped by z row block (k1, sp, kc); see the header comment.
 static void build_items(const BlkGeom& g, std::vector<std::vector<BlkItem>>* blocks) {
   const u64 nxp = (g.xb2 + 1) / 2, nyp = (g.yb2 + 1) / 2, nzp = (g.rb2 + 1) / 2;
-  const u64 pair_off = g.lc * g.row;
   for (u64 k1 = 0; k1 < g.rb1; k1++) {
     const u64 lo1 = sat_sub(k1 + 1, g.yb1), hi1 = std::min(k1 + 1, g.xb1);
     for (u64 sp = 0; sp < nzp; sp++)
@@ -372,7 +335,6 @@ static void build_items(const BlkGeom& g, std::vector<std::vector<BlkItem>>* blo
               }
           }
         }
-        (void)pair_off;
         if (!items.empty()) blocks->push_back(std::move(items));
       }
   }
@@ -401,7 +363,7 @@ static uint2 blk_entry(const BlkGeom& g, const BlkItem& it, int gi) {
 // different planes / slabs, whose strides are odd multiples of 16 bytes -> (almost) conflict-free LDS.128.
 // T teams share a lane's sequence round-robin (thread = team*lanes + lane).
 static bool build_fold_table(const BlkGeom& g, std::vector<uint2>* table, int* n_lo, int* n_hi) {
-  if (!blk_dense(g) || g.fold_b1 || g.octet) return false;
+  if (!blk_dense(g) || g.fold_b1) return false;
   const int D1 = (int)g.rb1, P = (int)(g.rb2 / 2);
   const int C1 = D1 / 2, DD = P / 2;
   const int nl = C1 * DD;
@@ -461,79 +423,27 @@ static bool build_fold_table(const BlkGeom& g, std::vector<uint2>* table, int* n
   return true;
 }
 
-// Octet table for single-plane slabs with 8 staged pairs: ONE column per octet (8 consecutive threads); the
-// lanes of an octet execute the same item on the 8 staged slab pairs g = 0..7, whose strides are odd multiples
-// of 16 bytes => every LDS.128 of a quarter-warp is conflict-free for ANY shape.  The z-block-major item list
-// of one slab pair is dealt evenly to the octets, so an octet changes output block (and flushes) only at the
-// few block boundaries inside its share, and keeps its block in registers from round to round.
-static void build_octet_table(const BlkGeom& g, std::vector<uint2>* table, int* n_lo, int* n_hi) {
-  std::vector<std::vector<BlkItem>> blocks;
-  build_items(g, &blocks);
-  std::vector<uint2> seq[2];
-  for (const auto& blk : blocks)
-    for (const BlkItem& it : blk) seq[it.kind].push_back(blk_entry(g, it, 0));
-  const int cols = g.bt / 8;
-  *n_lo = (int)((seq[0].size() + cols - 1) / cols);
-  *n_hi = (int)((seq[1].size() + cols - 1) / cols);
-  table->assign((size_t)std::max(*n_lo + *n_hi, 1) * cols, make_uint2(0u, 0u));
-  for (int kind = 0; kind < 2; kind++) {
-    const size_t T = seq[kind].size();
-    const size_t base = kind ? (size_t)*n_lo : 0;
-    for (int t = 0; t < cols; t++) {
-      size_t b = T * t / cols, e = T * (t + 1) / cols;
-      for (size_t i = b; i < e; i++) (*table)[(base + (i - b)) * cols + t] = seq[kind][i];
-    }
-  }
-}
-
-struct BlkPlan {
-  BufP table, units;
-  bool folded = false;
-  unsigned n_units = 0;
+struct BlkPlan : DfmaPlan {
   BlkP p;
   BlkGeom g;
 };
-struct BlkKey {
-  std::vector<u64> v;
-  bool operator<(const BlkKey& o) const { return v < o.v; }
-};
-using BlkCache = std::map<BlkKey, std::shared_ptr<BlkPlan>>;
-static BlkCache& blk_cache(Ctx& ctx) {
-  if (!ctx.blk_plans) ctx.blk_plans = std::make_shared<BlkCache>();
-  return *std::static_pointer_cast<BlkCache>(ctx.blk_plans);
-}
 
 template <int LT> static void blk_launch_lt(Ctx& ctx, const BlkPlan& pl, const BlkP& p) {
-  static size_t configured[2][64] = {};
-  const int ch = pl.g.lc > 1 ? 1 : 0;
-  if (configured[ch][ctx.device & 63] < pl.g.smem) {
-    if (ch) GTP_CUDA(cudaFuncSetAttribute(k_mul_blk<LT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
-    else GTP_CUDA(cudaFuncSetAttribute(k_mul_blk<LT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
-    configured[ch][ctx.device & 63] = pl.g.smem;
+  if (pl.g.lc > 1) {
+    allow_dyn_smem(k_mul_blk<LT, true>, ctx.device, pl.g.smem);
+    GTP_LAUNCH(ctx, (k_mul_blk<LT, true>), pl.n_units, BT, pl.g.smem, p);
+  } else {
+    allow_dyn_smem(k_mul_blk<LT, false>, ctx.device, pl.g.smem);
+    GTP_LAUNCH(ctx, (k_mul_blk<LT, false>), pl.n_units, BT, pl.g.smem, p);
   }
-  if (ch) GTP_LAUNCH(ctx, (k_mul_blk<LT, true>), pl.n_units, pl.g.bt, pl.g.smem, p);
-  else GTP_LAUNCH(ctx, (k_mul_blk<LT, false>), pl.n_units, pl.g.bt, pl.g.smem, p);
 }
 
 void launch_mul_blk(Ctx& ctx, const MulArgs& a) {
   BlkGeom g;
-  GTP_CHECK(blk_geom(a, &g, ctx.blk_octet), GTP_ERR_ARG, "blocked product kernel not applicable");
-  BlkKey key;
-  key.v.insert(key.v.end(), a.xs.begin(), a.xs.end());
-  key.v.insert(key.v.end(), a.ys.begin(), a.ys.end());
-  key.v.insert(key.v.end(), a.rs.begin(), a.rs.end());
-  key.v.push_back(a.row_begin);
-  key.v.push_back(a.row_step);
-  key.v.push_back(a.row_count);
-  key.v.push_back((ctx.blk_fold_tables ? 1 : 0) | (ctx.blk_octet ? 2 : 0));
-  key.v.insert(key.v.end(), a.rows.begin(), a.rows.end());
-  auto& cache = blk_cache(ctx);
-  std::shared_ptr<BlkPlan> pl;
-  auto it = cache.find(key);
-  if (it != cache.end()) {
-    pl = it->second;
-  } else {
-    pl = std::make_shared<BlkPlan>();
+  GTP_CHECK(blk_geom(a, &g), GTP_ERR_ARG, "blocked product kernel not applicable");
+  std::shared_ptr<void>& slot = dfma_plan_slot(ctx.blk_plans, a, 0);
+  if (!slot) {
+    auto pl = std::make_shared<BlkPlan>();
     pl->g = g;
     BlkP& p = pl->p;
     memset(&p, 0, sizeof(p));
@@ -560,14 +470,10 @@ void launch_mul_blk(Ctx& ctx, const MulArgs& a) {
     p.x_slab_sm = (unsigned)g.xslab; p.y_slab_sm = (unsigned)g.yslab;
     p.x_pair_off = p.y_pair_off = (unsigned)(g.lc * g.row);
     p.G = g.G;
-    // ---- item table: z-block major, then g, then the block's items; dealt evenly to the threads ----
+    // ---- item table: folded for dense cube slabs, else z-block major, then g, then the block's items, dealt evenly ----
     std::vector<uint2> table;
     int n_lo = 0, n_hi = 0;
-    p.octet = g.octet ? 1 : 0;
-    pl->folded = ctx.blk_fold_tables && build_fold_table(g, &table, &n_lo, &n_hi);
-    if (g.octet) {
-      build_octet_table(g, &table, &n_lo, &n_hi);
-    } else if (!pl->folded) {
+    if (!build_fold_table(g, &table, &n_lo, &n_hi)) {
       std::vector<std::vector<BlkItem>> blocks;
       build_items(g, &blocks);
       std::vector<uint2> seq[2];   // by kind
@@ -588,71 +494,27 @@ void launch_mul_blk(Ctx& ctx, const MulArgs& a) {
     }
     p.nsteps_lo = n_lo;
     p.nsteps = n_lo + n_hi;
-    // ---- work units ----
-    u64 n_slabs = a.row_count;
-    for (int d = 1; d < na; d++) n_slabs *= a.rs[d];
-    auto row_of = [&](u64 idx) -> u64 { return a.rows.empty() ? a.row_begin + idx * a.row_step : a.rows[idx]; };
-    struct U { unsigned ka, q0, q1, k0; };
-    std::vector<U> units;
-    std::vector<u64> boxes(n_slabs);
-    std::vector<unsigned> k0s(n_slabs, 0);
-    u64 total_pairs = 0;
-    for (u64 s = 0; s < n_slabs; s++) {
-      u64 rem = s, box = 1;
-      for (int d = na - 1; d >= 0; --d) {
-        u64 len = (d == 0) ? a.row_count : a.rs[d];
-        u64 idx = rem % len;
-        rem /= len;
-        u64 k = (d == 0) ? row_of(idx) : idx;
-        if (d == 0) k0s[s] = (unsigned)k;
-        u64 lo = sat_sub(k + 1, a.ys[d]), hi = std::min(k + 1, a.xs[d]);
-        box *= hi > lo ? hi - lo : 0;
-      }
-      boxes[s] = box;
-      total_pairs += box;
-    }
-    u64 slots = (u64)ctx.sm_count * (g.bt == 256 ? 1 : 2);
-    // at least 8 rounds per unit amortise its set-up -- unless that leaves resident-CTA slots empty (mid-size products)
-    const u64 min_chunk = total_pairs >= slots * 8 * (u64)g.G ? 8 * (u64)g.G : (u64)g.G;
-    u64 chunk = std::max<u64>(min_chunk, total_pairs / (slots * 16) + 1);
-    chunk = (chunk + g.G - 1) / g.G * g.G;   // whole rounds
-    for (u64 s = 0; s < n_slabs; s++) {
-      u64 box = boxes[s];
-      if (!box) continue;
-      u64 parts = (box + chunk - 1) / chunk;
-      u64 per = (box + parts - 1) / parts;
-      per = (per + g.G - 1) / g.G * g.G;
-      for (u64 q0 = 0; q0 < box; q0 += per) units.push_back({(unsigned)s, (unsigned)q0, (unsigned)std::min(box, q0 + per), k0s[s]});
-    }
-    std::stable_sort(units.begin(), units.end(), [](const U& x, const U& y) { return (x.q1 - x.q0) > (y.q1 - y.q0); });
-    pl->n_units = (unsigned)units.size();
-    std::vector<uint4> hu(units.size());
-    for (size_t i = 0; i < units.size(); i++) hu[i] = make_uint4(units[i].ka, units[i].q0, units[i].q1, units[i].k0);
-    pl->table = ctx.alloc(table.size() + 1);
-    pl->units = ctx.alloc(hu.size() * 2 + 1);
-    GTP_CUDA(cudaMemcpyAsync(pl->table->d, table.data(), table.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx.stream));
-    if (!hu.empty())
-      GTP_CUDA(cudaMemcpyAsync(pl->units->d, hu.data(), hu.size() * sizeof(uint4), cudaMemcpyHostToDevice, ctx.stream));
-    ctx.sync();
+    const Shape axs(a.xs.begin(), a.xs.begin() + na), ays(a.ys.begin(), a.ys.begin() + na), ars(a.rs.begin(), a.rs.begin() + na);
+    dfma_upload(ctx, pl.get(), table, dfma_units(a, axs, ays, ars, g.G, (u64)ctx.sm_count * 2));
     p.table = reinterpret_cast<const uint2*>(pl->table->d);
     p.units = reinterpret_cast<const uint4*>(pl->units->d);
-    if (cache.size() > 64) cache.clear();
-    cache[key] = pl;
+    slot = pl;
   }
-  BlkP p = pl->p;
+  const BlkPlan& pl = *std::static_pointer_cast<BlkPlan>(slot);
+  BlkP p = pl.p;
   p.x = a.x;
   p.y = a.y;
   p.out = a.out;
   u64 row_elems = 1;
   for (int d = 1; d < a.ndim; d++) row_elems *= a.rs[d];
   GTP_CUDA(cudaMemsetAsync(a.out, 0, a.row_count * row_elems * sizeof(double), ctx.stream));
-  if (pl->n_units == 0 || p.nsteps == 0) return;
-  switch ((int)pl->g.lt) {
-    case 8: blk_launch_lt<8>(ctx, *pl, p); break;
-    case 10: blk_launch_lt<10>(ctx, *pl, p); break;
-    case 12: blk_launch_lt<12>(ctx, *pl, p); break;
-    case 14: blk_launch_lt<14>(ctx, *pl, p); break;
-    case 16: blk_launch_lt<16>(ctx, *pl, p); break;
+  if (pl.n_units == 0 || p.nsteps == 0) return;
+  switch ((int)pl.g.lt) {
+    case 8: blk_launch_lt<8>(ctx, pl, p); break;
+    case 10: blk_launch_lt<10>(ctx, pl, p); break;
+    case 12: blk_launch_lt<12>(ctx, pl, p); break;
+    case 14: blk_launch_lt<14>(ctx, pl, p); break;
+    case 16: blk_launch_lt<16>(ctx, pl, p); break;
     default: throw Error(GTP_ERR_ARG, "unsupported chunk length");
   }
 }

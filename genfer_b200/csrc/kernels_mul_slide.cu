@@ -15,8 +15,6 @@
 // are folded (k <-> D-1-k on the plane axis and on the row pairs) so that every lane executes the same number of
 // steps in lockstep with conflict-free LDS.128, work units are LPT-sorted chunks of the jA box, partial rows meet in
 // HBM through RED.ADD.F64.
-#include <map>
-
 #include "kernels.cuh"
 
 namespace gtp {
@@ -52,10 +50,6 @@ constexpr unsigned SE_RELOAD = 1u << 26;
 constexpr unsigned SE_Z1 = 1u << 25;
 constexpr unsigned SE_UPPER = 1u << 27;   // tiled planes: the step feeds an output plane of the NEXT plane tile
 
-__device__ __forceinline__ void sl_cp16(void* smem, const void* gmem) {
-  unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
-}
 template <int LT> __device__ __forceinline__ void sl_load(double (&r)[LT], const double* __restrict__ p) {
 #pragma unroll
   for (int i = 0; i < LT; i += 2) {
@@ -189,8 +183,8 @@ __global__ void __launch_bounds__(ST, 3) k_mul_slide(const SlideP p) {
       for (int i = tid; i < n; i += ST) {
         int r = i / V2, c = i - r * V2;
         int pl = r / (int)p.prow, rr = r - pl * (int)p.prow;
-        sl_cp16(xs + pl * p.x_plane_sm + rr * p.row + 2 * c, gx + i);
-        sl_cp16(ys + pl * p.y_plane_sm + rr * p.row + 2 * c, gy + i);
+        cp_async16(xs + pl * p.x_plane_sm + rr * p.row + 2 * c, gx + i);
+        cp_async16(ys + pl * p.y_plane_sm + rr * p.row + 2 * c, gy + i);
       }
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
@@ -356,8 +350,8 @@ __global__ void __launch_bounds__(ST, 3) k_mul_slide16(const SlideP p) {
       constexpr int n = 16 * 16 * LT / 2;
       for (int i = tid; i < n; i += ST) {
         const int r = i >> 3, c = i & 7, pl = r >> 4, rr = r & 15;
-        sl_cp16(Xs + pl * p.x_plane_sm + rr * LT + 2 * c, gx + i);
-        sl_cp16(ys + pl * p.y_plane_sm + rr * LT + 2 * c, gy + i);
+        cp_async16(Xs + pl * p.x_plane_sm + rr * LT + 2 * c, gx + i);
+        cp_async16(ys + pl * p.y_plane_sm + rr * LT + 2 * c, gy + i);
       }
     }
     asm volatile("cp.async.wait_all;" ::: "memory");
@@ -435,17 +429,6 @@ struct SlideGeom {
   size_t smem;
 };
 
-static u64 sl_pick_chunk(u64 ltt) {
-  for (u64 lt : {16, 14, 12, 10, 8})
-    if (ltt % lt == 0) return lt;
-  return 0;
-}
-static u64 odd_groups(u64 doubles) {   // round up to an even number of doubles whose half is odd
-  doubles = (doubles + 1) / 2 * 2;
-  if ((doubles / 2) % 2 == 0) doubles += 2;
-  return doubles;
-}
-
 static void slide_smem_layout(SlideGeom* g) {
   g->row = g->lt;                                         // lockstep lanes differ by plane, not by row: no row padding
   g->xplane = odd_groups(g->D2 * g->lc * g->row);
@@ -462,7 +445,7 @@ static bool slide_geom(const Ctx& ctx, const MulArgs& a, SlideGeom* g) {
   if (a.xs[nd - 1] != ltt || a.ys[nd - 1] != ltt) return false;
   if (a.xs[nd - 3] != D1 || a.ys[nd - 3] != D1 || a.xs[nd - 2] != D2 || a.ys[nd - 2] != D2) return false;
   if (D1 % 2 != 0 || D2 % 4 != 0) return false;
-  const u64 lt = sl_pick_chunk(ltt);
+  const u64 lt = dfma_chunk(ltt);
   if (!lt) return false;
   for (int d = 0; d < nd; d++)
     if (a.xs[d] == 0 || a.ys[d] == 0 || a.rs[d] == 0) return false;
@@ -665,42 +648,20 @@ static void build_slide_table_tiled(const SlideGeom& g, std::vector<uint2>* tabl
     }
 }
 
-struct SlidePlan {
-  BufP table, units;
-  unsigned n_units = 0;
+struct SlidePlan : DfmaPlan {
   bool runs = false;   // k_mul_slide16 (no step table)
   SlideP p;
   SlideGeom g;
 };
-struct SlideKey {
-  std::vector<u64> v;
-  bool operator<(const SlideKey& o) const { return v < o.v; }
-};
-using SlideCache = std::map<SlideKey, std::shared_ptr<SlidePlan>>;
-static SlideCache& slide_cache(Ctx& ctx) {
-  if (!ctx.slide_plans) ctx.slide_plans = std::make_shared<SlideCache>();
-  return *std::static_pointer_cast<SlideCache>(ctx.slide_plans);
-}
 
 template <int LT> static void slide_launch_lt(Ctx& ctx, const SlidePlan& pl, const SlideP& p) {
-  static size_t configured[2][64] = {};
-  const int ch = pl.g.lc > 1 ? 1 : 0;
-  if (configured[ch][ctx.device & 63] < pl.g.smem) {
-    if (ch) GTP_CUDA(cudaFuncSetAttribute(k_mul_slide<LT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
-    else GTP_CUDA(cudaFuncSetAttribute(k_mul_slide<LT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
-    configured[ch][ctx.device & 63] = pl.g.smem;
+  if (pl.g.lc > 1) {
+    allow_dyn_smem(k_mul_slide<LT, true>, ctx.device, pl.g.smem);
+    GTP_LAUNCH(ctx, (k_mul_slide<LT, true>), pl.n_units, pl.g.threads, pl.g.smem, p);
+  } else {
+    allow_dyn_smem(k_mul_slide<LT, false>, ctx.device, pl.g.smem);
+    GTP_LAUNCH(ctx, (k_mul_slide<LT, false>), pl.n_units, pl.g.threads, pl.g.smem, p);
   }
-  if (ch) GTP_LAUNCH(ctx, (k_mul_slide<LT, true>), pl.n_units, pl.g.threads, pl.g.smem, p);
-  else GTP_LAUNCH(ctx, (k_mul_slide<LT, false>), pl.n_units, pl.g.threads, pl.g.smem, p);
-}
-
-static void slide_launch_runs(Ctx& ctx, const SlidePlan& pl, const SlideP& p) {
-  static size_t configured[64] = {};
-  if (configured[ctx.device & 63] < pl.g.smem) {
-    GTP_CUDA(cudaFuncSetAttribute(k_mul_slide16, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.g.smem));
-    configured[ctx.device & 63] = pl.g.smem;
-  }
-  GTP_LAUNCH(ctx, k_mul_slide16, pl.n_units, pl.g.threads, pl.g.smem, p);
 }
 
 void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
@@ -709,23 +670,9 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
   // whole 16^3 slabs run on k_mul_slide16 (ctx.slide_runs = false: the table-driven kernel, for A/B measurements)
   const bool runs = ctx.slide_runs && g.nt == 1 && g.D1 == 16 && g.D2 == 16 && g.lt == 16 && g.lc == 1 && g.G == 1 && g.threads == ST;
   if (runs) g.smem += 3 * 16 * sizeof(double);   // the zero rows of the padding pairs
-  SlideKey key;
-  key.v.insert(key.v.end(), a.xs.begin(), a.xs.end());
-  key.v.insert(key.v.end(), a.ys.begin(), a.ys.end());
-  key.v.insert(key.v.end(), a.rs.begin(), a.rs.end());
-  key.v.push_back(g.T1);
-  key.v.push_back(runs ? 1 : 0);
-  key.v.push_back(a.row_begin);
-  key.v.push_back(a.row_step);
-  key.v.push_back(a.row_count);
-  key.v.insert(key.v.end(), a.rows.begin(), a.rows.end());
-  auto& cache = slide_cache(ctx);
-  std::shared_ptr<SlidePlan> pl;
-  auto it = cache.find(key);
-  if (it != cache.end()) {
-    pl = it->second;
-  } else {
-    pl = std::make_shared<SlidePlan>();
+  std::shared_ptr<void>& slot = dfma_plan_slot(ctx.slide_plans, a, g.T1 << 1 | (runs ? 1 : 0));
+  if (!slot) {
+    auto pl = std::make_shared<SlidePlan>();
     pl->g = g;
     pl->runs = runs;
     SlideP& p = pl->p;
@@ -771,77 +718,32 @@ void launch_mul_slide(Ctx& ctx, const MulArgs& a) {
     else if (tiled) build_slide_table_tiled(g, &table, &p.nsteps_lo, &p.nsteps);
     else build_slide_table(g, &table, &p.nsteps_lo, &p.nsteps);
     p.nsteps += p.nsteps_lo;
-    // ---- work units (as in kernels_mul_blk.cu) ----
-    u64 n_slabs = a.row_count;
-    for (int d = 1; d < na; d++) n_slabs *= ars[d];
-    auto row_of = [&](u64 idx) -> u64 { return a.rows.empty() ? a.row_begin + idx * a.row_step : a.rows[idx]; };
-    struct U { unsigned ka, q0, q1, k0; };
-    std::vector<U> units;
-    std::vector<u64> boxes(n_slabs);
-    std::vector<unsigned> k0s(n_slabs, 0);
-    u64 total_pairs = 0;
-    for (u64 s = 0; s < n_slabs; s++) {
-      u64 rem = s, box = 1;
-      for (int d = na - 1; d >= 0; --d) {
-        u64 len = (d == 0) ? a.row_count : ars[d];
-        u64 idx = rem % len;
-        rem /= len;
-        u64 k = (d == 0) ? row_of(idx) : idx;
-        if (d == 0) k0s[s] = (unsigned)k;
-        u64 lo = sat_sub(k + 1, ays[d]), hi = std::min(k + 1, axs[d]);
-        box *= hi > lo ? hi - lo : 0;
-      }
-      boxes[s] = box;
-      total_pairs += box;
-    }
-    u64 slots = (u64)ctx.sm_count * g.ctas;
-    // at least 8 rounds per unit amortise its set-up -- unless that leaves resident-CTA slots empty (mid-size products)
-    const u64 min_chunk = total_pairs >= slots * 8 * (u64)g.G ? 8 * (u64)g.G : (u64)g.G;
-    u64 chunk = std::max<u64>(min_chunk, total_pairs / (slots * 16) + 1);
-    chunk = (chunk + g.G - 1) / g.G * g.G;
-    for (u64 s = 0; s < n_slabs; s++) {
-      u64 box = boxes[s];
-      if (!box) continue;
-      u64 parts = (box + chunk - 1) / chunk;
-      u64 per = (box + parts - 1) / parts;
-      per = (per + g.G - 1) / g.G * g.G;
-      for (u64 q0 = 0; q0 < box; q0 += per) units.push_back({(unsigned)s, (unsigned)q0, (unsigned)std::min(box, q0 + per), k0s[s]});
-    }
-    std::stable_sort(units.begin(), units.end(), [](const U& x, const U& y) { return (x.q1 - x.q0) > (y.q1 - y.q0); });
-    pl->n_units = (unsigned)units.size();
-    std::vector<uint4> hu(units.size());
-    for (size_t i = 0; i < units.size(); i++) hu[i] = make_uint4(units[i].ka, units[i].q0, units[i].q1, units[i].k0);
-    pl->table = ctx.alloc(table.size() + 1);
-    pl->units = ctx.alloc(hu.size() * 2 + 1);
-    if (!table.empty())
-      GTP_CUDA(cudaMemcpyAsync(pl->table->d, table.data(), table.size() * sizeof(uint2), cudaMemcpyHostToDevice, ctx.stream));
-    if (!hu.empty())
-      GTP_CUDA(cudaMemcpyAsync(pl->units->d, hu.data(), hu.size() * sizeof(uint4), cudaMemcpyHostToDevice, ctx.stream));
-    ctx.sync();
+    dfma_upload(ctx, pl.get(), table, dfma_units(a, axs, ays, ars, g.G, (u64)ctx.sm_count * g.ctas));
     p.table = reinterpret_cast<const uint2*>(pl->table->d);
     p.units = reinterpret_cast<const uint4*>(pl->units->d);
-    if (cache.size() > 64) cache.clear();
-    cache[key] = pl;
+    slot = pl;
   }
-  SlideP p = pl->p;
+  const SlidePlan& pl = *std::static_pointer_cast<SlidePlan>(slot);
+  SlideP p = pl.p;
   p.x = a.x;
   p.y = a.y;
   p.out = a.out;
   u64 row_elems = 1;
   for (int d = 1; d < a.ndim; d++) row_elems *= a.rs[d];
   GTP_CUDA(cudaMemsetAsync(a.out, 0, a.row_count * row_elems * sizeof(double), ctx.stream));
-  if (pl->n_units == 0) return;
-  if (pl->runs) {
-    slide_launch_runs(ctx, *pl, p);
+  if (pl.n_units == 0) return;
+  if (pl.runs) {
+    allow_dyn_smem(k_mul_slide16, ctx.device, pl.g.smem);
+    GTP_LAUNCH(ctx, k_mul_slide16, pl.n_units, pl.g.threads, pl.g.smem, p);
     return;
   }
   if (p.nsteps == 0) return;
-  switch ((int)pl->g.lt) {
-    case 8: slide_launch_lt<8>(ctx, *pl, p); break;
-    case 10: slide_launch_lt<10>(ctx, *pl, p); break;
-    case 12: slide_launch_lt<12>(ctx, *pl, p); break;
-    case 14: slide_launch_lt<14>(ctx, *pl, p); break;
-    case 16: slide_launch_lt<16>(ctx, *pl, p); break;
+  switch ((int)pl.g.lt) {
+    case 8: slide_launch_lt<8>(ctx, pl, p); break;
+    case 10: slide_launch_lt<10>(ctx, pl, p); break;
+    case 12: slide_launch_lt<12>(ctx, pl, p); break;
+    case 14: slide_launch_lt<14>(ctx, pl, p); break;
+    case 16: slide_launch_lt<16>(ctx, pl, p); break;
     default: throw Error(GTP_ERR_ARG, "unsupported chunk length");
   }
 }

@@ -656,7 +656,6 @@ static std::shared_ptr<WaveTables> wave_tables(Ctx& ctx, const std::vector<u64>&
 template <int OP, bool EXACT>
 static bool wave_launch(Ctx& ctx, WaveP& p, unsigned want_ctas, size_t smem) {
   static int coop[64] = {};           // 0 unknown, 1 yes, -1 no
-  static size_t configured[64] = {};
   int& c = coop[ctx.device & 63];
   if (c == 0) {
     int v = 0;
@@ -665,10 +664,7 @@ static bool wave_launch(Ctx& ctx, WaveP& p, unsigned want_ctas, size_t smem) {
   }
   if (c < 0) return false;
   auto* fn = k_rec_wave<OP, EXACT>;
-  if (configured[ctx.device & 63] < smem) {
-    GTP_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   // static + dynamic may pass 48 KB
-    configured[ctx.device & 63] = smem;
-  }
+  allow_dyn_smem(fn, ctx.device, smem);   // static + dynamic may pass 48 KB
   int per_sm = 0;
   GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, WV_T, smem));
   if (per_sm < 1) return false;

@@ -70,8 +70,8 @@ uint64_t gtp_ctx_launch_count(gtp_ctx* ctx);
 /* tuning knob: 0 = always use the reference-order product kernel (bit-identical products, Horner loops and 2-axis log / exp;
  * general N-D division and N-D log stay tolerance-level: their wavefront / descending-row summation order is not the reference's),
  * 1 = pick the fastest applicable kernel (default: DFMA kernels from 2^20 MACs), 2 = use the DFMA kernels even for
- * tiny products (tests).  A/B bits: +4 evenly dealt instead of folded item tables (blocked kernel), +8 octet tables
- * (experimental), +16 sliding kernel off, +32 / +64 force the plane-tiled sliding plan with 4 / 8 planes per slab,
+ * tiny products (tests).  A/B bits: +4 and +8 are ignored (retired variants of the blocked kernel's item tables),
+ * +16 sliding kernel off, +32 / +64 force the plane-tiled sliding plan with 4 / 8 planes per slab,
  * +128 mul_linear as the reference's composition instead of the one-pass kernel, +256 small-operand stencil kernel off,
  * +512 stencil kernel with one instead of four coefficients per thread, +1024 device-resident N-D div / exp / log
  * recurrences off (host loops of product launches), +2048 fused Horner loop of subst_var off (three launches per step),

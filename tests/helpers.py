@@ -37,6 +37,17 @@ def assert_close(g, o, rtol=RTOL, atol_scale=None):
     assert not bad.any(), f"max rel err {np.max(err / np.maximum(np.abs(oa), 1e-300))}\n gpu={ga}\n ref={oa}"
 
 
+def small_ints(shape, seed):
+    """Operands of integers 0..3: every product and partial sum of a DFMA product kernel is then an exact integer in f64,
+    whatever the summation or RED.ADD meeting order, so a missed or repeated multiply-add shows as a bit difference."""
+    return np.random.default_rng(seed).integers(0, 4, size=shape).astype(np.float64)
+
+
+def assert_bits(got, ref):
+    diff = np.flatnonzero(got.view(np.uint64) != ref.view(np.uint64))
+    assert diff.size == 0, f"{diff.size} coefficients differ, first at flat {diff[0]}: {got.flat[diff[0]]} != {ref.flat[diff[0]]}"
+
+
 from genfer_b200.synth import splitmix64, synth_pgf, synth_uniform  # noqa: E402,F401
 
 

@@ -8,7 +8,7 @@
 import numpy as np
 import pytest
 
-from helpers import RTOL, synth_pgf, synth_uniform
+from helpers import RTOL, assert_bits, small_ints, synth_pgf, synth_uniform
 
 pytestmark = pytest.mark.gpu
 
@@ -23,8 +23,9 @@ def ctx():
     c.close()
 
 
-def gpu_mul_raw(ctx, x, y, rshape, rows=None, fast=True):
-    """Calls gtp_mul_rows_raw through the C ABI on torch-owned device buffers."""
+def gpu_mul_raw(ctx, x, y, rshape, rows=None, fast=True, row_list=None):
+    """Calls gtp_mul_rows_raw (rows = (begin, step, count), default all) or gtp_mul_rowlist_raw (row_list) through the
+    C ABI on torch-owned device buffers."""
     import torch
     ctx.set_fast_mul(fast)
     xd = torch.from_numpy(np.ascontiguousarray(x)).cuda()
@@ -33,9 +34,14 @@ def gpu_mul_raw(ctx, x, y, rshape, rows=None, fast=True):
         begin, step, count = 0, 1, rshape[0]
     else:
         begin, step, count = rows
+    if row_list is not None:
+        count = len(row_list)
     out = torch.full((count,) + tuple(rshape[1:]), float("nan"), dtype=torch.float64, device="cuda")
     torch.cuda.synchronize()
-    ctx.mul_rows_raw(x.shape, xd.data_ptr(), y.shape, yd.data_ptr(), rshape, begin, step, count, out.data_ptr())
+    if row_list is not None:
+        ctx.mul_rowlist_raw(x.shape, xd.data_ptr(), y.shape, yd.data_ptr(), rshape, row_list, out.data_ptr())
+    else:
+        ctx.mul_rows_raw(x.shape, xd.data_ptr(), y.shape, yd.data_ptr(), rshape, begin, step, count, out.data_ptr())
     ctx.synchronize()
     ctx.set_fast_mul(1)
     return out.cpu().numpy()
@@ -217,6 +223,30 @@ def test_blocked_kernel_ragged_match_oracle(ctx, xs, ys, rs):
     ref = O.mul_raw(x, y, rs)
     got = gpu_mul_raw(ctx, x, y, rs, fast=2)
     np.testing.assert_allclose(got, ref, rtol=1e-11, atol=1e-12)
+
+
+BLK_ROW_SHAPES = [((12,) * 4,) * 3,                                   # folded item table (dense cube slabs)
+                  ((16,) * 3,) * 3,                                   # evenly dealt table (single-plane slabs)
+                  ((5, 7, 9, 16), (6, 4, 9, 16), (8, 9, 12, 16))]     # evenly dealt, odd row counts, unequal boxes
+
+
+@pytest.mark.parametrize("xs,ys,rs", BLK_ROW_SHAPES)
+def test_blocked_kernel_row_shards_are_exact(ctx, xs, ys, rs):
+    """Row shards through the 2x2-blocked kernel (mode 18 forces the DFMA kernels and switches the sliding one off), as
+    partitioned multi-GPU products send them: cyclic rows (gtp_mul_rows_raw) and a folded-cyclic row list
+    (gtp_mul_rowlist_raw).  Small-integer operands: bit for bit against the oracle."""
+    from oracle import oracle as O
+    from genfer_b200.partition import rows_for_rank
+    x, y = small_ints(xs, 61), small_ints(ys, 62)
+    ref = O.mul_raw(x, y, rs)
+    ctx.set_fast_mul(18)
+    kind = ctx.mul_kernel_kind(xs, ys, rs)
+    ctx.set_fast_mul(1)
+    assert kind == 2
+    cyclic = (1, 3, len(range(1, rs[0], 3)))
+    assert_bits(gpu_mul_raw(ctx, x, y, rs, rows=cyclic, fast=18), ref[1::3])
+    folded = rows_for_rank(rs[0], 2, 1)
+    assert_bits(gpu_mul_raw(ctx, x, y, rs, row_list=folded, fast=18), ref[folded])
 
 
 @pytest.mark.parametrize("n,d,world", [(3, 16, 2), (4, 8, 4), (3, 16, 8), (4, 16, 8)])

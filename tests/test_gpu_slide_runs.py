@@ -8,6 +8,8 @@ step-table kernel) and requires both to be bit-identical to the oracle.
 import numpy as np
 import pytest
 
+from helpers import assert_bits, small_ints
+
 pytestmark = pytest.mark.gpu
 
 SLIDE_TABLE = 1 << 19   # gtp_ctx_set_fast_mul bit: whole 16^3 slabs on the step-table kernel
@@ -25,10 +27,6 @@ def ctx():
     yield c
     genfer_b200.set_default_context(None)
     c.close()
-
-
-def small_ints(shape, seed):
-    return np.random.default_rng(seed).integers(0, 4, size=shape).astype(np.float64)
 
 
 def device_product(ctx, mode, x, y, rshape, rows=None, row_list=None):
@@ -51,11 +49,6 @@ def device_product(ctx, mode, x, y, rshape, rows=None, row_list=None):
     finally:
         ctx.set_fast_mul(1)
     return out.cpu().numpy()
-
-
-def assert_bits(got, ref):
-    diff = np.flatnonzero(got.view(np.uint64) != ref.view(np.uint64))
-    assert diff.size == 0, f"{diff.size} coefficients differ, first at flat {diff[0]}: {got.flat[diff[0]]} != {ref.flat[diff[0]]}"
 
 
 @pytest.fixture(scope="module")
