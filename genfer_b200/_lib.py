@@ -17,6 +17,7 @@ MAX_NDIM = 24
 STATUS = {0: "GTP_OK", 1: "GTP_ERR_INDEX", 2: "GTP_ERR_SHAPE", 3: "GTP_ERR_OOM", 4: "GTP_ERR_CUDA", 5: "GTP_ERR_ARG"}
 
 u64p = C.POINTER(C.c_uint64)
+u32p = C.POINTER(C.c_uint32)
 f64p = C.POINTER(C.c_double)
 vp = C.c_void_p
 vpp = C.POINTER(C.c_void_p)
@@ -155,6 +156,14 @@ _SIGS = {
     "gtu_subst": (C.c_int, [vp, vp, vp, vpp]),
     "gtu_taylor_expansion_of_coeff": (C.c_int, [vp, vp, C.c_uint64, vpp]),
     "gtu_eq": (C.c_int, [vp, vp, vp, intp]),
+    "gtu_program_create": (C.c_int, [vp, vpp]),
+    "gtu_program_free": (None, [vp, vp]),
+    "gtu_program_constant": (C.c_int, [vp, vp, C.c_double, u32p]),
+    "gtu_program_var": (C.c_int, [vp, vp, C.c_double, C.c_uint64, u32p]),
+    "gtu_program_from_coefficients": (C.c_int, [vp, vp, f64p, C.c_uint64, u32p]),
+    "gtu_program_op": (C.c_int, [vp, vp, C.c_int, C.c_uint32, C.c_uint32, C.c_uint32, u32p]),
+    "gtu_program_slot": (C.c_int, [vp, C.c_uint32, intp, u64p]),
+    "gtu_program_run": (C.c_int, [vp, vp, u32p, C.c_int, f64p]),
 }
 
 SYMBOLS = tuple(_SIGS)

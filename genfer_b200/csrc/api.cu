@@ -1299,14 +1299,7 @@ int gtp_gather_axis(gtp_ctx* c, const gtp_poly* a, uint64_t v, uint64_t count, d
     u64 stride = v < a->shape.size() ? stride_of(a->shape, v) : 0;
     BufP tmp = c->alloc(count);
     launch_gather_strided(*c, a->ptr(), stride, len, count, tmp->d);
-    if (c->gather_cap < count) {
-      if (c->gather_host) cudaFreeHost(c->gather_host);
-      c->gather_host = nullptr;
-      c->gather_cap = 0;
-      GTP_CUDA(cudaMallocHost((void**)&c->gather_host, std::max<u64>(count, 1024) * sizeof(double)));
-      c->gather_cap = std::max<u64>(count, 1024);
-    }
-    GTP_CUDA(cudaMemcpyAsync(c->gather_host, tmp->d, count * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    GTP_CUDA(cudaMemcpyAsync(c->host_staging(count), tmp->d, count * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
     c->sync();
     std::memcpy(out, c->gather_host, count * sizeof(double));
   });

@@ -246,6 +246,17 @@ struct Ctx {
   BufP alloc(u64 n_doubles);
   BufP alloc_host_visible(const double* vals, int n);   // n <= 2: a scalar-pool slot holding vals (nullptr: pool unavailable)
   void sync() { GTP_CUDA(cudaStreamSynchronize(stream)); }
+  // gather_host with room for n doubles; grows it (the old block must not be in use by a pending copy)
+  double* host_staging(u64 n) {
+    if (gather_cap < n) {
+      if (gather_host) cudaFreeHost(gather_host);
+      gather_host = nullptr;
+      gather_cap = 0;
+      GTP_CUDA(cudaMallocHost((void**)&gather_host, std::max<u64>(n, 1024) * sizeof(double)));
+      gather_cap = std::max<u64>(n, 1024);
+    }
+    return gather_host;
+  }
 };
 
 // Cached data-dependent classification of a handle (multivariate_taylor.rs:262-294, :643-655)

@@ -87,30 +87,75 @@ struct GpuBackend {
     return out;
   }
 
-  // ---- TaylorExpansion<F64> (univariate_taylor.rs) for the symbolic mode: gtu_* -----------------------------------
-  struct UniHandle {
+  // ---- TaylorExpansion<F64> (univariate_taylor.rs) for the symbolic mode: a gtu_program per evaluation -----------------
+  // Every operator records into the current program; the variant and order of each value are known on the host at once.
+  // The first coefficient read of an evaluation runs the program (one launch, one read-back of the whole value); further
+  // reads of that value come from the host copy.  The next value recorded after a run starts a new program.
+  struct Program {
     gtp_ctx* c;
-    gtu_series* s;
-    UniHandle(gtp_ctx* c_, gtu_series* s_) : c(c_), s(s_) {}
-    ~UniHandle() { if (s) gtu_free(c, s); }
-    UniHandle(const UniHandle&) = delete;
-    UniHandle& operator=(const UniHandle&) = delete;
+    gtu_program* p;
+    bool ran = false;
+    uint32_t read_slot = 0;     // the value whose coefficients `host` holds (valid once ran)
+    std::vector<double> host;
+    Program(gtp_ctx* c_, gtu_program* p_) : c(c_), p(p_) {}
+    ~Program() { gtu_program_free(c, p); }
+    Program(const Program&) = delete;
+    Program& operator=(const Program&) = delete;
   };
-  using Uni = std::shared_ptr<UniHandle>;
-  Uni uwrap(gtu_series* s) const { return std::make_shared<UniHandle>(ctx, s); }
-  Uni uni_constant(double x) { gtu_series* o; check(gtu_constant(ctx, x, &o)); return uwrap(o); }
-  Uni uni_var(double x, size_t order) { gtu_series* o; check(gtu_var(ctx, x, order, &o)); return uwrap(o); }
-#define GFE_UBIN(name, fn) Uni name(const Uni& a, const Uni& b) { gtu_series* o; check(fn(ctx, a->s, b->s, &o)); return uwrap(o); }
-  GFE_UBIN(uni_add, gtu_add) GFE_UBIN(uni_mul, gtu_mul) GFE_UBIN(uni_div, gtu_div)
-#undef GFE_UBIN
-  Uni uni_exp(const Uni& a) { gtu_series* o; check(gtu_exp(ctx, a->s, &o)); return uwrap(o); }
-  Uni uni_log(const Uni& a) { gtu_series* o; check(gtu_log(ctx, a->s, &o)); return uwrap(o); }
-  Uni uni_pow(const Uni& a, uint32_t e) { gtu_series* o; check(gtu_pow(ctx, a->s, e, &o)); return uwrap(o); }
-  Uni uni_max(const Uni& a, const Uni& b) {   // :219-224: constants only
-    if (!gtu_is_constant(a->s) || !gtu_is_constant(b->s)) throw gfe::EvalError("Maximum can only be applied to constant Taylor expansions.");
-    return uni_constant(scalar_max(uni_coeff(a, 0), uni_coeff(b, 0)));
+  struct Uni {
+    std::shared_ptr<Program> prog;
+    uint32_t slot = 0;
+    bool is_const = true;
+    uint64_t n = 1;
+  };
+  std::shared_ptr<Program> cur;
+  gtu_program* recording() {
+    if (!cur || cur->ran) {
+      gtu_program* p;
+      check(gtu_program_create(ctx, &p));
+      cur = std::make_shared<Program>(ctx, p);
+    }
+    return cur->p;
   }
-  double uni_coeff(const Uni& a, size_t order) { double x; check(gtu_coeff(ctx, a->s, order, &x)); return x; }
+  Uni uni_slot(uint32_t slot) {
+    Uni u{cur, slot, true, 1};
+    int is_c = 0;
+    check(gtu_program_slot(cur->p, slot, &is_c, &u.n));
+    u.is_const = is_c != 0;
+    if (u.is_const) u.n = 1;
+    return u;
+  }
+  Uni uni_op(int op, const Uni& a, const Uni* b, uint32_t e = 0) {
+    gtu_program* p = recording();
+    if (a.prog != cur || (b && b->prog != cur)) throw gfe::EvalError("univariate value used after its program ran");
+    uint32_t s;
+    check(gtu_program_op(ctx, p, op, a.slot, b ? b->slot : 0, e, &s));
+    return uni_slot(s);
+  }
+  Uni uni_constant(double x) { uint32_t s; check(gtu_program_constant(ctx, recording(), x, &s)); return uni_slot(s); }
+  Uni uni_var(double x, size_t order) { uint32_t s; check(gtu_program_var(ctx, recording(), x, order, &s)); return uni_slot(s); }
+  Uni uni_add(const Uni& a, const Uni& b) { return uni_op(GTU_ADD, a, &b); }
+  Uni uni_mul(const Uni& a, const Uni& b) { return uni_op(GTU_MUL, a, &b); }
+  Uni uni_div(const Uni& a, const Uni& b) { return uni_op(GTU_DIV, a, &b); }
+  Uni uni_exp(const Uni& a) { return uni_op(GTU_EXP, a, nullptr); }
+  Uni uni_log(const Uni& a) { return uni_op(GTU_LOG, a, nullptr); }
+  Uni uni_pow(const Uni& a, uint32_t e) { return uni_op(GTU_POW, a, nullptr, e); }
+  Uni uni_max(const Uni& a, const Uni& b) {   // :219-224: constants only
+    if (!a.is_const || !b.is_const) throw gfe::EvalError("Maximum can only be applied to constant Taylor expansions.");
+    return uni_op(GTU_MAX, a, &b);
+  }
+  double uni_coeff(const Uni& a, size_t order) {   // gtu_coeff (:25-36) of the value
+    if (a.is_const && order != 0) return 0.0;
+    if (!a.is_const && order >= a.n) throw gfe::EvalError("libgenfer_taylor: coeff: index out of bounds");
+    Program& pr = *a.prog;
+    if (!pr.ran || pr.read_slot != a.slot) {
+      pr.host.resize(a.n);
+      check(gtu_program_run(ctx, pr.p, &a.slot, 1, pr.host.data()));
+      pr.ran = true;
+      pr.read_slot = a.slot;
+    }
+    return pr.host[a.is_const ? 0 : order];
+  }
 };
 
 // Interval<F64> as the evaluator sees it (src/interval.rs): constructible from an f64 constant (a point interval); the

@@ -272,9 +272,47 @@ void uni_mul(Ctx& ctx, const double* u, const double* w, double* r, u64 order); 
 void uni_div(Ctx& ctx, const double* u, bool u_const, const double* w, double* r, u64 order);  // :409-436
 void uni_exp(Ctx& ctx, const double* c, double* r, u64 order);                            // :153-164
 void uni_log(Ctx& ctx, const double* c, double* r, u64 order);                            // :172-185
-// r[i] = op(a[i or 0], b[i or 0]) element-wise family for the Constant/Polynomial combinations
+// r[i] = op(a[i or 0], b[i or 0]) element-wise family for the Constant/Polynomial combinations (op: UniEw)
 void uni_ew(Ctx& ctx, int op, const double* a, bool a_bcast, const double* b, bool b_bcast, double* r, u64 n);
 void uni_teoc(Ctx& ctx, const double* in, double* out, u64 n, u64 len);                   // :78-87
 void uni_factorial_times(Ctx& ctx, const double* in, u64 order, double* out);             // :47-51
+
+// uni_ew's operations
+enum UniEw : int {
+  UEW_ADD = 0, UEW_SUB = 1, UEW_MUL = 2, UEW_DIV = 3, UEW_NEG = 4,
+  UEW_ADD_FIRST = 5,    // r = a; r[0] += b
+  UEW_SUB_FIRST = 6,    // r = a; r[0] -= b
+  UEW_RSUB_FIRST = 7,   // r = -a; r[0] += b
+  UEW_MAX = 8,          // a > b ? a : b (Constants only)
+};
+// The kernel that runs one univariate op
+enum UniKind : int { UK_EW = 0, UK_MUL, UK_DIV, UK_EXP, UK_LOG, UK_SCALAR_EXP, UK_SCALAR_LOG };
+// What an op (GTU_ADD ... GTU_MAX) does to operands of the given variants and lengths (n: 1 for a Constant): the result's
+// variant and length and the kernel that computes it.  The kernel's operands are (a, b), or (b, a) when `swap`; a_b / b_b
+// broadcast element 0 of the kernel's first / second operand (UK_DIV: a_b = the dividend is a Constant).  Throws the
+// reference's errors: GTP_ERR_INDEX for Max of a Polynomial, GTP_ERR_ARG for a quotient above order 2048.
+struct UniPlan {
+  bool is_const = true;
+  u64 n = 1;
+  int kind = UK_EW;
+  int ew = 0;
+  bool swap = false, a_b = false, b_b = false;
+};
+UniPlan uni_plan(int op, bool a_const, u64 a_n, bool b_const, u64 b_n);
+// runs a plan with the per-op kernels; b may be null for unary ops
+void uni_run(Ctx& ctx, const UniPlan& p, const double* a, const double* b, double* r);
+
+// One instruction of a univariate program (k_uni_program): a plan with its kernel operands resolved to arena offsets
+constexpr unsigned UNI_NONE = 0xffffffffu;
+struct UniIns {
+  unsigned a, b, r;   // arena offsets (doubles) of the kernel's first and second operand (UNI_NONE: none) and of the result
+  unsigned n;         // result length
+  unsigned char kind, ew, a_b, b_b;
+  unsigned pad;
+};
+static_assert(sizeof(UniIns) == 24, "UniIns is packed into a double-aligned upload");
+// ins / lvl / outs / arena are device pointers; lvl has nlevels * nwarps + 1 entries, outs n_out (src, len, dst) triples
+void uni_program_launch(Ctx& ctx, const UniIns* ins, const unsigned* lvl, int nlevels, int nwarps, const unsigned* outs, int n_out,
+                        double* arena);
 
 }  // namespace gtp

@@ -476,3 +476,82 @@ class TaylorExpansion:
         if not self._h or not self.ctx.h:
             return "TaylorExpansion(<released>)"
         return f"TaylorExpansion({'Constant' if self.is_const() else 'Polynomial'}, {self.coeffs().tolist()})"
+
+
+GTU_ADD, GTU_SUB, GTU_MUL, GTU_DIV, GTU_NEG, GTU_EXP, GTU_LOG, GTU_POW, GTU_MAX = range(9)
+
+
+class UniProgram:
+    """A DAG of univariate TaylorExpansion<F64> ops recorded on the host and run by one kernel launch (gtu_program_*).
+
+    Each op means exactly the TaylorExpansion operator of the same name, with the same bits; its errors are raised when it
+    is recorded.  ``run(*slots)`` runs every recorded op and returns the slots' coefficients as numpy arrays (one element
+    for a Constant)."""
+
+    def __init__(self, ctx: Optional[Context] = None):
+        self.ctx = ctx or default_context()
+        self._h = C.c_void_p()
+        self.ctx.check(self.ctx.lib.gtu_program_create(self.ctx.h, C.byref(self._h)))
+
+    def __del__(self):
+        try:
+            if self._h and self.ctx.h:
+                self.ctx.lib.gtu_program_free(self.ctx.h, self._h)
+        except Exception:
+            pass
+
+    def _slot(self, fn: str, *args) -> "UniSlot":
+        s = C.c_uint32()
+        self.ctx.check(getattr(self.ctx.lib, fn)(self.ctx.h, self._h, *args, C.byref(s)))
+        return UniSlot(self, s.value)
+
+    def constant(self, x: float) -> "UniSlot": return self._slot("gtu_program_constant", float(x))
+    def var(self, x: float, order: int) -> "UniSlot": return self._slot("gtu_program_var", float(x), order)
+
+    def from_coefficients(self, xs) -> "UniSlot":
+        a = np.ascontiguousarray(xs, dtype=np.float64)
+        return self._slot("gtu_program_from_coefficients", a.ctypes.data_as(_lib.f64p), a.shape[0])
+
+    def op(self, op: int, a: "UniSlot", b: Optional["UniSlot"] = None, exp: int = 0) -> "UniSlot":
+        for s in (a, b):
+            if s is not None and s.program is not self:
+                raise ValueError("slot of another program")
+        return self._slot("gtu_program_op", op, a.index, b.index if b is not None else 0, exp)
+
+    def run(self, *slots: "UniSlot"):
+        for s in slots:
+            if s.program is not self:
+                raise ValueError("slot of another program")
+        lens = [1 if s.is_const() else s.order() for s in slots]
+        out = np.empty(max(sum(lens), 1), dtype=np.float64)
+        idx = (C.c_uint32 * max(len(slots), 1))(*[s.index for s in slots])
+        self.ctx.check(self.ctx.lib.gtu_program_run(self.ctx.h, self._h, idx, len(slots), out.ctypes.data_as(_lib.f64p)))
+        return np.split(out[:sum(lens)], np.cumsum(lens)[:-1]) if slots else []
+
+
+class UniSlot:
+    """A value of a :class:`UniProgram`: supports ``+ - * /``, unary ``-``, ``exp``, ``log``, ``pow`` and ``max``."""
+
+    __slots__ = ("program", "index")
+
+    def __init__(self, program: UniProgram, index: int):
+        self.program = program
+        self.index = index
+
+    def _info(self):
+        c, n = C.c_int(), C.c_uint64()
+        self.program.ctx.check(self.program.ctx.lib.gtu_program_slot(self.program._h, self.index, C.byref(c), C.byref(n)))
+        return bool(c.value), int(n.value)
+
+    def is_const(self) -> bool: return self._info()[0]
+    def order(self) -> int: return self._info()[1]
+
+    def __add__(self, o): return self.program.op(GTU_ADD, self, o)
+    def __sub__(self, o): return self.program.op(GTU_SUB, self, o)
+    def __mul__(self, o): return self.program.op(GTU_MUL, self, o)
+    def __truediv__(self, o): return self.program.op(GTU_DIV, self, o)
+    def __neg__(self): return self.program.op(GTU_NEG, self)
+    def exp(self): return self.program.op(GTU_EXP, self)
+    def log(self): return self.program.op(GTU_LOG, self)
+    def pow(self, e: int): return self.program.op(GTU_POW, self, exp=e)
+    def max(self, o): return self.program.op(GTU_MAX, self, o)

@@ -226,6 +226,31 @@ int gtu_subst(gtp_ctx* ctx, const gtu_series* a, const gtu_series* subst, gtu_se
 int gtu_taylor_expansion_of_coeff(gtp_ctx* ctx, const gtu_series* a, uint64_t n, gtu_series** out); /* :69-89 */
 int gtu_eq(gtp_ctx* ctx, const gtu_series* a, const gtu_series* b, int* out);         /* derive(PartialEq) :8 */
 
+/* ---- univariate programs: a DAG of TaylorExpansion<F64> ops recorded on the host, run by one kernel launch ------------
+ * Every slot is a value of the program.  Inputs (constant / var / from_coefficients) are copied at record time; an op
+ * records a new slot whose variant (Constant / Polynomial) and order are known at once (gtu_program_slot).  Each op means
+ * exactly the gtu_* call of the same name -- the same variant and order rules, the same errors, raised when it is
+ * recorded (GTP_ERR_ARG for a bad slot or a quotient above order 2048, GTP_ERR_INDEX for GTU_MAX of a Polynomial) -- and
+ * the same bits in every coefficient.  GTU_POW records the binary exponentiation of gtu_pow (`exp` is the exponent; `b`
+ * is ignored, as it is for the unary ops); GTU_MAX is F64::max (x > y ? x : y) of two Constants.
+ * gtu_program_run uploads the program in one host-to-device copy, runs every recorded op in one launch of a single CTA
+ * (independent ops on different warps), reads the `outputs` back in one device-to-host copy and synchronises.  `out`
+ * receives the outputs' coefficients one after another (1 double for a Constant, the order for a Polynomial).  A program
+ * may be run again, and recorded into further between runs. */
+typedef struct gtu_program gtu_program;
+typedef enum gtu_op {
+  GTU_ADD = 0, GTU_SUB = 1, GTU_MUL = 2, GTU_DIV = 3, GTU_NEG = 4, GTU_EXP = 5, GTU_LOG = 6, GTU_POW = 7, GTU_MAX = 8
+} gtu_op;
+int gtu_program_create(gtp_ctx* ctx, gtu_program** out);
+void gtu_program_free(gtp_ctx* ctx, gtu_program* p);
+int gtu_program_constant(gtp_ctx* ctx, gtu_program* p, double x, uint32_t* slot);
+int gtu_program_var(gtp_ctx* ctx, gtu_program* p, double x, uint64_t order, uint32_t* slot);
+int gtu_program_from_coefficients(gtp_ctx* ctx, gtu_program* p, const double* xs, uint64_t n, uint32_t* slot);
+int gtu_program_op(gtp_ctx* ctx, gtu_program* p, int op, uint32_t a, uint32_t b, uint32_t exp, uint32_t* slot);
+/* the slot's variant and order (gtu_is_constant / gtu_order: GTP_UNBOUNDED for a Constant); GTP_ERR_ARG for a bad slot */
+int gtu_program_slot(const gtu_program* p, uint32_t slot, int* is_constant, uint64_t* n);
+int gtu_program_run(gtp_ctx* ctx, gtu_program* p, const uint32_t* outputs, int n_outputs, double* out);
+
 /* ---- host evaluator: an SGCL program end to end (SURVEY 8 f1) ------------------------------------ */
 /* Plays the role of the reference's `genfer file.sgcl` for the default f64 Taylor mode -- run() / run_program::<F64>
  * (src/main.rs:108-227): parse (src/parser.rs), translate to a generating function (src/semantics/gf.rs), simplify
@@ -239,7 +264,8 @@ int gtu_eq(gtp_ctx* ctx, const gtu_series* a, const gtu_series* b, int* out);   
  *            the GenFun is evaluated unsimplified in this mode;
  *            8 = -s / --symbolic (src/main.rs:196-209, src/symbolic.rs): the generating function becomes ONE univariate
  *            computation DAG on the host (symbolic Taylor coefficients, evaluator/symbolic.hpp) and that DAG is evaluated
- *            over TaylorExpansion<F64> through gtu_* (probs_symbolic / moments_symbolic :238-299); F64 only
+ *            over TaylorExpansion<F64> as a gtu_program: one launch per evaluation (the rest, the moments and the
+ *            probabilities: 3 launches, 2 with --no-probs) (probs_symbolic / moments_symbolic :238-299); F64 only
  *   unroll : --unroll (reference default 8; only used by `while`)
  * On error (parse error, or anything the reference would panic on) returns GTP_ERR_INDEX and copies the message
  * into `err`.  The report is byte-compatible with the reference's stdout under --no-timing. */

@@ -11,6 +11,7 @@ pub const GTP_UNBOUNDED: u64 = u64::MAX; // usize::MAX on 64-bit targets
 #[repr(C)] pub struct gtp_ctx { _p: [u8; 0] }
 #[repr(C)] pub struct gtp_poly { _p: [u8; 0] }
 #[repr(C)] pub struct gtu_series { _p: [u8; 0] }
+#[repr(C)] pub struct gtu_program { _p: [u8; 0] }
 #[repr(C)] pub struct gtp_sgcl_result { _p: [u8; 0] }
 #[repr(C)] pub struct gti_poly { _p: [u8; 0] }
 
@@ -104,6 +105,14 @@ extern "C" {
     pub fn gtu_subst(ctx: *mut gtp_ctx, a: *const gtu_series, subst: *const gtu_series, out: *mut *mut gtu_series) -> c_int;
     pub fn gtu_taylor_expansion_of_coeff(ctx: *mut gtp_ctx, a: *const gtu_series, n: u64, out: *mut *mut gtu_series) -> c_int;
     pub fn gtu_eq(ctx: *mut gtp_ctx, a: *const gtu_series, b: *const gtu_series, out: *mut c_int) -> c_int;
+    pub fn gtu_program_create(ctx: *mut gtp_ctx, out: *mut *mut gtu_program) -> c_int;
+    pub fn gtu_program_free(ctx: *mut gtp_ctx, p: *mut gtu_program);
+    pub fn gtu_program_constant(ctx: *mut gtp_ctx, p: *mut gtu_program, x: f64, slot: *mut u32) -> c_int;
+    pub fn gtu_program_var(ctx: *mut gtp_ctx, p: *mut gtu_program, x: f64, order: u64, slot: *mut u32) -> c_int;
+    pub fn gtu_program_from_coefficients(ctx: *mut gtp_ctx, p: *mut gtu_program, xs: *const f64, n: u64, slot: *mut u32) -> c_int;
+    pub fn gtu_program_op(ctx: *mut gtp_ctx, p: *mut gtu_program, op: c_int, a: u32, b: u32, exp: u32, slot: *mut u32) -> c_int;
+    pub fn gtu_program_slot(p: *const gtu_program, slot: u32, is_constant: *mut c_int, n: *mut u64) -> c_int;
+    pub fn gtu_program_run(ctx: *mut gtp_ctx, p: *mut gtu_program, outputs: *const u32, n_outputs: c_int, out: *mut f64) -> c_int;
     pub fn gtp_run_sgcl(ctx: *mut gtp_ctx, source: *const c_char, limit: i64, flags: c_int, unroll: u64, out: *mut *mut gtp_sgcl_result, err: *mut c_char, err_cap: usize) -> c_int;
     pub fn gtp_sgcl_free(r: *mut gtp_sgcl_result);
     pub fn gtp_sgcl_report(r: *const gtp_sgcl_result) -> *const c_char;
