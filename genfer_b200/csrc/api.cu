@@ -1396,7 +1396,9 @@ int gtp_mul_kernel_kind(gtp_ctx* c, int ndim, const uint64_t* xs, const uint64_t
   m.ys = to_shape(ys, ndim);
   m.rs = to_shape(rs, ndim);
   m.row_count = m.rs.empty() ? 1 : m.rs[0];
-  return mul_plan_kind(*c, m);
+  int kind = 0;
+  wrap(c, [&] { kind = mul_kernel_kind(*c, m); });   // planning queries the device (cooperative-kernel occupancy)
+  return kind;
 }
 int gtp_fp64_peak_probe(gtp_ctx* c, int kind, int iters, double* flops, double* ms) {
   return wrap(c, [&] { fp64_peak_probe(*c, kind, iters, flops, ms); });

@@ -1,6 +1,8 @@
 // Launcher declarations for the device kernels of libgenfer_taylor (sm_100a).
 #pragma once
+#include <algorithm>
 #include <mutex>
+#include <tuple>
 
 #include "common.hpp"
 
@@ -33,6 +35,38 @@ inline void allow_dyn_smem(const void* fn, int device, size_t bytes) {
   cur = bytes;
 }
 template <class F> void allow_dyn_smem(F* fn, int device, size_t bytes) { allow_dyn_smem((const void*)fn, device, bytes); }
+
+// Cooperative launches (persistent kernels with a grid barrier: every CTA must be resident).  Resident CTAs per SM of `fn`
+// with `block` threads and `smem` bytes of dynamic shared memory on `device` (the current device), after allow_dyn_smem;
+// 0 when the device has no cooperative launch or the kernel cannot be resident.  The record is per (kernel, device, block,
+// smem) and shared by all contexts, which may live on different threads.
+inline int coop_ctas_per_sm(const void* fn, int device, int block, size_t smem) {
+  static std::mutex mu;
+  static std::map<std::tuple<const void*, int, int, size_t>, int> known;
+  std::lock_guard<std::mutex> lock(mu);
+  const auto key = std::make_tuple(fn, device, block, smem);
+  auto it = known.find(key);
+  if (it != known.end()) return it->second;
+  int coop = 0, per_sm = 0;
+  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device);
+  if (coop) {
+    allow_dyn_smem(fn, device, smem);
+    GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, block, smem));
+  }
+  return known[key] = std::max(per_sm, 0);
+}
+// Launches `fn` cooperatively on the context's stream with one parameter struct, counted and timed as GTP_LAUNCH does
+// (`tag`: its name in the GTP_LAUNCH_HIST census).
+inline void coop_launch(Ctx& ctx, const void* fn, unsigned grid, int block, size_t smem, void* params, const char* tag) {
+  void* args[] = {params};
+  const double t0 = ctx.hist ? Ctx::now() : 0.0;
+  GTP_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(block), args, smem, ctx.stream));
+  ctx.launches++;
+  if (ctx.hist) {
+    (*ctx.hist)[tag]++;
+    ctx.t_launch += Ctx::now() - t0;
+  }
+}
 
 // 16-byte global -> shared copy that bypasses L1 (the DFMA product kernels stage their slabs with it)
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
@@ -195,8 +229,10 @@ struct MulArgs {
   double sign = 1.0;
 };
 void launch_mul(Ctx& ctx, const MulArgs& a);
+// The product kernel launch_mul runs for `a` (its plan, nothing launched): 0 the reference-order family (reference-order
+// kernel, small-operand products, axis convolution: all bit-exact), 2 / 3 the blocked / sliding DFMA kernel, 6 / 7 the same
+// after zero-extending odd extents.
 int mul_kernel_kind(const Ctx& ctx, const MulArgs& a);
-int mul_plan_kind(const Ctx& ctx, const MulArgs& a);   // incl. the zero-extended plans (6 / 7)
 double mul_macs(const Shape& xs, const Shape& ys, const Shape& rs);
 double args_macs(const MulArgs& a);   // MACs of the rows this launch computes
 // Products below this many MACs stay on the reference-order kernel (bit-exact, and launch-bound anyway); above it the
@@ -228,6 +264,19 @@ struct DfmaPlan {
 std::shared_ptr<void>& dfma_plan_slot(std::shared_ptr<void>& cache, const MulArgs& a, u64 extra);
 // Copies the step table and the units to new device arrays of `pl` (empty arrays are not copied) and waits for the copy.
 void dfma_upload(Ctx& ctx, DfmaPlan* pl, const std::vector<uint2>& table, const std::vector<uint4>& units);
+
+// The terms of a small operand (at most 32 coefficients, extents <= 255) in a product or a Horner step: coefficient sidx[t]
+// pairs with the big operand at k - m[t] (m over the `ne` effective axes `eff`; the small operand has extent 1 on every
+// other axis).  Sorted in the reference's visiting order, ascending X index: ascending m when the small operand is X,
+// descending m (`descending`) when it is Y; group_start[t] marks the first term of each group of equal outer offsets.
+constexpr int SMALL_MAXT = 32, SMALL_MAXE = 8;
+struct SmallTerms {
+  int nt;
+  unsigned char m[SMALL_MAXT][SMALL_MAXE];   // zero beyond the effective axes
+  unsigned short sidx[SMALL_MAXT];
+  unsigned char group_start[SMALL_MAXT];
+};
+SmallTerms small_terms(const Shape& ss, const int* eff, int ne, bool descending);
 
 void fp64_peak_probe(Ctx& ctx, int kind, int iters, double* flops, double* ms);
 

@@ -47,6 +47,15 @@ struct HornerP {
   unsigned* bar;
 };
 
+// the term table of the substitution (or of a product's small operand)
+static void set_terms(HornerP* p, const SmallTerms& st) {
+  static_assert(sizeof(p->m) == sizeof(st.m), "HornerP holds the term table as it is built");
+  p->nt = st.nt;
+  memcpy(p->m, st.m, sizeof(p->m));
+  memcpy(p->sidx, st.sidx, sizeof(p->sidx));
+  memcpy(p->group_start, st.group_start, sizeof(p->group_start));
+}
+
 __global__ void __launch_bounds__(HN_T) k_horner(const __grid_constant__ HornerP p) {
   __shared__ double s_sv[HN_MAXT];
   __shared__ long long s_delta[HN_MAXT];   // offset of res[k - m_t] relative to res[k], for this step's strides
@@ -758,25 +767,36 @@ __global__ void __launch_bounds__(HD_T, (NT <= 4 ? (MODE == 0 ? 4 : 3) : (NT <= 
   }
 }
 
-static bool launch_direct_variant(Ctx& ctx, const HornerP& p, int add_mode, const unsigned* final_shape, u64 final_total, const char* tag) {
+// One cooperative launch of a Horner kernel: the kernel, its geometry and its parameters
+struct HornerLaunch {
+  const void* fn;
+  unsigned grid;
+  int block;
+  size_t smem;
+  const char* tag;   // its name in the GTP_LAUNCH_HIST census
+  union {
+    HornerP h;
+    HornerDirectP direct;
+    HornerBulkP bulk;
+  } params;
+};
+
+void launch_horner_plan(Ctx& ctx, const HornerLaunch& pl) {
+  coop_launch(ctx, pl.fn, pl.grid, pl.block, pl.smem, const_cast<void*>((const void*)&pl.params), pl.tag);
+}
+
+// Plans k_horner_direct for the steps of `p`; false: outside its domain.
+static bool plan_direct_variant(const Ctx& ctx, const HornerP& p, int add_mode, const unsigned* final_shape, u64 final_total, const char* tag,
+                                HornerLaunch* pl) {
   if (!ctx.use_direct || p.ne < 2) return false;
   const unsigned L_final = final_shape[p.ne - 1];
   if ((L_final < 48 && p.ne < 3) || final_total < ctx.direct_min) return false;   // short rows need a second row axis to walk blocks
   if (add_mode == 0 && L_final < 192 && !ctx.direct_products_all) return false;   // plain products: the gather kernel wins on shorter rows
-  HornerDirectP dp;
+  HornerDirectP& dp = pl->params.direct;
   memset(&dp, 0, sizeof(dp));
   dp.h = p;
   dp.add_mode = add_mode;
-  static int coop[64] = {};
-  int& c = coop[ctx.device & 63];
-  if (c == 0) {
-    int vv = 0;
-    cudaDeviceGetAttribute(&vv, cudaDevAttrCooperativeLaunch, ctx.device);
-    c = vv ? 1 : -1;
-  }
-  if (c < 0) return false;
   const void* fn;
-  int bucket;
   // uniform group size (terms per group): 1 or 2 for the usual substitutions, else 0 = read the group starts at run time
   int gsz = 0;
   {
@@ -796,46 +816,37 @@ static bool launch_direct_variant(Ctx& ctx, const HornerP& p, int add_mode, cons
   }
 #define HD_PICK3(NT_, U_, GS_) (add_mode == 0 ? (const void*)k_horner_direct<NT_, U_, 0, GS_> : (add_mode == 1 ? (const void*)k_horner_direct<NT_, U_, 1, GS_> : (const void*)k_horner_direct<NT_, U_, 2, GS_>))
 #define HD_PICK(NT_, U_) (gsz == 2 ? HD_PICK3(NT_, U_, 2) : (gsz == 1 ? HD_PICK3(NT_, U_, 1) : HD_PICK3(NT_, U_, 0)))
-  if (p.nt <= 2) { fn = HD_PICK(2, 4); bucket = 0; }
-  else if (p.nt <= 4) { fn = HD_PICK(4, 2); bucket = 1; }
-  else if (p.nt <= 8) { fn = HD_PICK(8, 2); bucket = 2; }
-  else if (p.nt <= 16) { gsz = 0; fn = HD_PICK3(16, 1, 0); bucket = 3; }
-  else { gsz = 0; fn = HD_PICK3(32, 1, 0); bucket = 4; }
+  if (p.nt <= 2) fn = HD_PICK(2, 4);
+  else if (p.nt <= 4) fn = HD_PICK(4, 2);
+  else if (p.nt <= 8) fn = HD_PICK(8, 2);
+  else if (p.nt <= 16) fn = HD_PICK3(16, 1, 0);
+  else fn = HD_PICK3(32, 1, 0);
 #undef HD_PICK
 #undef HD_PICK3
-  bucket = (bucket * 3 + add_mode) * 3 + gsz;
-  static int per_sm_cached[45][64] = {};
-  int& per_sm = per_sm_cached[bucket][ctx.device & 63];
-  if (per_sm == 0) {
-    GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, HD_T, 0));
-    if (per_sm < 1) per_sm = -1;
-  }
-  if (per_sm < 0) return false;
+  const int per_sm = coop_ctas_per_sm(fn, ctx.device, HD_T, 0);
+  if (per_sm == 0) return false;
   // rows per warp item at the final shape; mid-size tensors are barrier-bound (fewer CTAs), HBM-sized ones want loads in flight
   unsigned W = 32;
   while (W > 1 && (W >> 1) >= L_final) W >>= 1;
   const u64 items = (final_total / L_final + (32 / W) - 1) / (32 / W);
   const int want_per_sm = final_total >= (1u << 21) ? ctx.direct_ctas : (final_total >= (1u << 18) ? 2 : 1);
   const int ctas_per_sm = std::max(1, std::min(per_sm, want_per_sm));
-  const unsigned grid = (unsigned)std::max<u64>(1, std::min<u64>((items + HD_T / 32 - 1) / (HD_T / 32), (u64)ctas_per_sm * ctx.sm_count));
-  void* args[] = {(void*)&dp};
-  const double t0 = ctx.hist ? Ctx::now() : 0.0;
-  GTP_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(HD_T), args, 0, ctx.stream));
-  ctx.launches++;
-  if (ctx.hist) {
-    (*ctx.hist)[tag]++;
-    ctx.t_launch += Ctx::now() - t0;
-  }
+  pl->fn = fn;
+  pl->grid = (unsigned)std::max<u64>(1, std::min<u64>((items + HD_T / 32 - 1) / (HD_T / 32), (u64)ctas_per_sm * ctx.sm_count));
+  pl->block = HD_T;
+  pl->smem = 0;
+  pl->tag = tag;
   return true;
 }
 
-// Fills the group tables from the (sorted) terms of `p` and launches k_horner_rows; false: outside its domain.
-static bool launch_rows_variant(Ctx& ctx, const HornerP& p, int add_mode, const unsigned* final_shape, u64 final_total, const char* tag) {
+// Fills the group tables from the (sorted) terms of `p` and plans k_horner_rows; false: outside its domain.
+static bool plan_rows_variant(const Ctx& ctx, const HornerP& p, int add_mode, const unsigned* final_shape, u64 final_total, const char* tag,
+                              HornerLaunch* pl) {
   if (!ctx.use_bulk || p.ne < 2) return false;
   const unsigned L_final = final_shape[p.ne - 1];
   if (L_final < 16 || L_final > 2048 || final_total < (1u << 18)) return false;
   if ((reinterpret_cast<uintptr_t>(p.res0) & 15u) || (reinterpret_cast<uintptr_t>(p.buf[0]) & 15u) || (reinterpret_cast<uintptr_t>(p.buf[1]) & 15u)) return false;
-  HornerBulkP bp;
+  HornerBulkP& bp = pl->params.bulk;
   memset(&bp, 0, sizeof(bp));
   bp.h = p;
   bp.add_mode = add_mode;
@@ -872,34 +883,20 @@ static bool launch_rows_variant(Ctx& ctx, const HornerP& p, int add_mode, const 
   bp.R = R;
   const size_t smem = (size_t)HB_NS * R * ng * bp.slot * sizeof(double);
   if (smem > 200 * 1024) return false;
-  static int coop[64] = {};
-  int& c = coop[ctx.device & 63];
-  if (c == 0) {
-    int vv = 0;
-    cudaDeviceGetAttribute(&vv, cudaDevAttrCooperativeLaunch, ctx.device);
-    c = vv ? 1 : -1;
-  }
-  if (c < 0) return false;
   const void* fn;
   if (p.nt <= 2) fn = (const void*)k_horner_rows<2>;
   else if (p.nt <= 4) fn = (const void*)k_horner_rows<4>;
   else if (p.nt <= 8) fn = (const void*)k_horner_rows<8>;
   else if (p.nt <= 16) fn = (const void*)k_horner_rows<16>;
   else fn = (const void*)k_horner_rows<32>;
-  allow_dyn_smem(fn, ctx.device, smem);
-  int per_sm = 0;
-  GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, HB_T, smem));
-  if (per_sm < 1) return false;
+  const int per_sm = coop_ctas_per_sm(fn, ctx.device, HB_T, smem);
+  if (per_sm == 0) return false;
   const u64 nsr = final_total / block;
-  const unsigned grid = (unsigned)std::max<u64>(1, std::min<u64>((nsr + R - 1) / R, (u64)std::min(per_sm, 4) * ctx.sm_count));
-  void* args[] = {(void*)&bp};
-  const double t0 = ctx.hist ? Ctx::now() : 0.0;
-  GTP_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(HB_T), args, smem, ctx.stream));
-  ctx.launches++;
-  if (ctx.hist) {
-    (*ctx.hist)[tag]++;
-    ctx.t_launch += Ctx::now() - t0;
-  }
+  pl->fn = fn;
+  pl->grid = (unsigned)std::max<u64>(1, std::min<u64>((nsr + R - 1) / R, (u64)std::min(per_sm, 4) * ctx.sm_count));
+  pl->block = HB_T;
+  pl->smem = smem;
+  pl->tag = tag;
   return true;
 }
 
@@ -917,14 +914,17 @@ bool launch_horner(Ctx& ctx, const double* self, const Shape& self_shape, u64 v,
   for (int a = 0; a < nd; a++) slice[a] = std::min(self_shape[a], d[a]);
   slice[v] = 1;
   // effective axes: the non-unit axes of res; every axis that can become non-unit must already be one
-  std::vector<int> eff;
+  int eff[HN_MAXE], ne = 0;
   for (int a = 0; a < nd; a++) {
-    if (rshape[a] > 1) eff.push_back(a);
-    else if (sshape[a] > 1 || slice[a] > 1) return false;
+    if (rshape[a] > 1) {
+      if (ne == HN_MAXE) return false;
+      eff[ne++] = a;
+    } else if (sshape[a] > 1 || slice[a] > 1) {
+      return false;
+    }
     if (sshape[a] > d[a] || sshape[a] > 255) return false;
   }
-  const int ne = (int)eff.size();
-  if (ne < 1 || ne > HN_MAXE) return false;
+  if (ne < 1) return false;
   // final shape (the same recurrence the kernel runs) and overflow checks
   Shape cur = rshape;
   const u64 nsteps = i_top + 1;
@@ -943,11 +943,8 @@ bool launch_horner(Ctx& ctx, const double* self, const Shape& self_shape, u64 v,
   HornerP p;
   memset(&p, 0, sizeof(p));
   p.ne = ne;
-  Shape selfst(nd, 1), sst(nd, 1);
-  for (int a = nd - 2; a >= 0; --a) {
-    selfst[a] = selfst[a + 1] * self_shape[a + 1];
-    sst[a] = sst[a + 1] * sshape[a + 1];
-  }
+  Shape selfst(nd, 1);
+  for (int a = nd - 2; a >= 0; --a) selfst[a] = selfst[a + 1] * self_shape[a + 1];
   for (int e = 0; e < ne; e++) {
     const int a = eff[e];
     p.d[e] = d[a] >= 0xffffffffull ? 0xffffffffu : (unsigned)d[a];
@@ -957,27 +954,8 @@ bool launch_horner(Ctx& ctx, const double* self, const Shape& self_shape, u64 v,
     p.shape0[e] = (unsigned)rshape[a];
   }
   p.self_vstr = (long long)selfst[v];
-  // terms of subst in the reference's visiting order: X = res index ascending <=> m descending (lexicographic)
-  struct Term { std::vector<unsigned> m; u64 idx; };
-  std::vector<Term> terms;
-  for (u64 lin = 0; lin < ns; lin++) {
-    u64 rem = lin;
-    std::vector<unsigned> full(nd);
-    for (int a = nd - 1; a >= 0; --a) { full[a] = (unsigned)(rem % sshape[a]); rem /= sshape[a]; }
-    Term t;
-    t.idx = lin;
-    for (int e = 0; e < ne; e++) t.m.push_back(full[eff[e]]);
-    terms.push_back(t);
-  }
-  std::sort(terms.begin(), terms.end(), [](const Term& x, const Term& y) { return x.m > y.m; });
-  p.nt = (int)terms.size();
-  for (int t = 0; t < p.nt; t++) {
-    for (int e = 0; e < ne; e++) p.m[t][e] = (unsigned char)terms[t].m[e];
-    p.sidx[t] = (unsigned short)terms[t].idx;
-    bool new_group = t == 0;
-    for (int e = 0; e < ne - 1 && !new_group; e++) new_group = terms[t].m[e] != terms[t - 1].m[e];
-    p.group_start[t] = new_group ? 1 : 0;
-  }
+  // terms of subst in the reference's visiting order: X = res index ascending <=> m descending
+  set_terms(&p, small_terms(sshape, eff, ne, true));
   p.self = self;
   p.subst = subst;
   p.res0 = res;
@@ -990,52 +968,36 @@ bool launch_horner(Ctx& ctx, const double* self, const Shape& self_shape, u64 v,
   p.buf[0] = b0->d;
   p.buf[1] = b1 ? b1->d : b0->d;
   p.bar = reinterpret_cast<unsigned*>(bar->d);
-  *out_buf = ((nsteps - 1) & 1) ? b1 : b0;
-  *out_shape = cur;
-  {
-    unsigned fs[HN_MAXE];
-    for (int e = 0; e < ne; e++) fs[e] = (unsigned)cur[eff[e]];
-    if (launch_direct_variant(ctx, p, p.slice_scalar ? 2 : 1, fs, final_total, "k_horner_direct")) return true;
-    if (launch_rows_variant(ctx, p, p.slice_scalar ? 2 : 1, fs, final_total, "k_horner_rows")) return true;
+  unsigned fs[HN_MAXE];
+  for (int e = 0; e < ne; e++) fs[e] = (unsigned)cur[eff[e]];
+  const int add_mode = p.slice_scalar ? 2 : 1;
+  HornerLaunch pl;
+  if (!plan_direct_variant(ctx, p, add_mode, fs, final_total, "k_horner_direct", &pl) &&
+      !plan_rows_variant(ctx, p, add_mode, fs, final_total, "k_horner_rows", &pl)) {
+    const int per_sm = coop_ctas_per_sm((const void*)k_horner, ctx.device, HN_T, 0);
+    if (per_sm == 0) return false;
+    const u64 want = (final_total + HN_T - 1) / HN_T;
+    // small and mid-size tensors are barrier-bound (a step is ~1 us of L2 traffic): one CTA per SM keeps the barrier short;
+    // HBM-sized tensors want every resident CTA for loads in flight
+    const int ctas_per_sm = final_total >= (1u << 21) ? std::min(per_sm, 4) : (final_total >= (1u << 18) ? std::min(per_sm, 2) : 1);
+    pl.params.h = p;
+    pl.fn = (const void*)k_horner;
+    pl.grid = (unsigned)std::max<u64>(1, std::min<u64>(want, (u64)ctas_per_sm * ctx.sm_count));
+    pl.block = HN_T;
+    pl.smem = 0;
+    pl.tag = "k_horner";
   }
-  static int coop[64] = {};
-  int& c = coop[ctx.device & 63];
-  if (c == 0) {
-    int vv = 0;
-    cudaDeviceGetAttribute(&vv, cudaDevAttrCooperativeLaunch, ctx.device);
-    c = vv ? 1 : -1;
-  }
-  if (c < 0) return false;
-  static int per_sm_cached[64] = {};
-  int& per_sm = per_sm_cached[ctx.device & 63];
-  if (per_sm == 0) {
-    GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_horner, HN_T, 0));
-    if (per_sm < 1) per_sm = -1;
-  }
-  if (per_sm < 0) return false;
-  const u64 want = (final_total + HN_T - 1) / HN_T;
-  // small and mid-size tensors are barrier-bound (a step is ~1 us of L2 traffic): one CTA per SM keeps the barrier short;
-  // HBM-sized tensors want every resident CTA for loads in flight
-  const int ctas_per_sm = final_total >= (1u << 21) ? std::min(per_sm, 4) : (final_total >= (1u << 18) ? std::min(per_sm, 2) : 1);
-  const unsigned grid = (unsigned)std::max<u64>(1, std::min<u64>(want, (u64)ctas_per_sm * ctx.sm_count));
-  void* args[] = {(void*)&p};
-  const double t0 = ctx.hist ? Ctx::now() : 0.0;
-  GTP_CUDA(cudaLaunchCooperativeKernel((const void*)k_horner, dim3(grid), dim3(HN_T), args, 0, ctx.stream));
-  ctx.launches++;
-  if (ctx.hist) {
-    (*ctx.hist)["k_horner"]++;
-    ctx.t_launch += Ctx::now() - t0;
-  }
+  launch_horner_plan(ctx, pl);
   *out_buf = ((nsteps - 1) & 1) ? b1 : b0;
   *out_shape = cur;
   return true;
 }
 
-// The plain small-operand product (launch_mul_stencil's case, kernels_mul.cu) on the row-staged kernel: one "step" without
-// the Add.  false: outside the domain (the caller continues with the gather kernels).
-bool launch_stencil_rows(Ctx& ctx, const MulArgs& a) {
+// The plain small-operand product (the small-operand route of kernels_mul.cu) as one step of the Horner kernels without
+// the Add.  Null: outside their domain (the caller goes on to the stencil kernels).
+std::shared_ptr<const HornerLaunch> plan_small_rows(const Ctx& ctx, const MulArgs& a) {
   const int nd = a.ndim;
-  if (a.accumulate || !a.rows.empty() || nd < 2 || a.row_begin != 0 || a.row_step != 1 || a.row_count != a.rs[0]) return false;
+  if (a.accumulate || !a.rows.empty() || nd < 2 || a.row_begin != 0 || a.row_step != 1 || a.row_count != a.rs[0]) return nullptr;
   {  // cheap rejections first: this sits on the path of every small-operand product, most of them tiny
     u64 total = 1, last = 1;
     for (int d = 0; d < nd; d++) {
@@ -1044,32 +1006,30 @@ bool launch_stencil_rows(Ctx& ctx, const MulArgs& a) {
     }
     const bool direct = ctx.direct_products && ctx.use_direct && total >= ctx.direct_min && (last >= 192 || ctx.direct_products_all);
     const bool bulk = ctx.bulk_products && ctx.use_bulk && total >= (1u << 18);
-    if (!direct && !bulk) return false;
+    if (!direct && !bulk) return nullptr;
   }
   const u64 nx = prod(a.xs), ny = prod(a.ys);
   const bool small_is_x = nx <= ny;
   const Shape& ss = small_is_x ? a.xs : a.ys;
   const Shape& bs = small_is_x ? a.ys : a.xs;
   const u64 ns = std::min(nx, ny);
-  if (ns < 1 || ns > (u64)HN_MAXT) return false;
-  std::vector<int> eff;
+  if (ns < 1 || ns > (u64)HN_MAXT) return nullptr;
+  int eff[HN_MAXE], ne = 0;
   for (int d = 0; d < nd; d++) {
     if (a.rs[d] == 1) {
-      if (a.xs[d] != 1 || a.ys[d] != 1) return false;
+      if (a.xs[d] != 1 || a.ys[d] != 1) return nullptr;
       continue;
     }
-    if (a.rs[d] > bs[d] + ss[d] - 1 || ss[d] > 255) return false;   // no rows / columns beyond the product's own extent
-    eff.push_back(d);
+    if (a.rs[d] > bs[d] + ss[d] - 1 || ss[d] > 255) return nullptr;   // no rows / columns beyond the product's own extent
+    if (ne == HN_MAXE) return nullptr;
+    eff[ne++] = d;
   }
-  const int ne = (int)eff.size();
-  if (ne < 2 || ne > HN_MAXE) return false;
+  if (ne < 2) return nullptr;
   const u64 total = prod(a.rs);
-  if (total >= (1ull << 31) || prod(bs) >= (1ull << 31)) return false;
+  if (total >= (1ull << 31) || prod(bs) >= (1ull << 31)) return nullptr;
   HornerP p;
   memset(&p, 0, sizeof(p));
   p.ne = ne;
-  Shape sst(nd, 1);
-  for (int d = nd - 2; d >= 0; --d) sst[d] = sst[d + 1] * ss[d + 1];
   unsigned fs[HN_MAXE];
   for (int e = 0; e < ne; e++) {
     const int d = eff[e];
@@ -1079,32 +1039,7 @@ bool launch_stencil_rows(Ctx& ctx, const MulArgs& a) {
     p.shape0[e] = (unsigned)bs[d];
     fs[e] = (unsigned)a.rs[d];
   }
-  struct Term { std::vector<unsigned> m; u64 idx; };
-  std::vector<Term> terms;
-  for (u64 lin = 0; lin < ns; lin++) {
-    u64 rem = lin;
-    std::vector<unsigned> full(nd);
-    for (int d = nd - 1; d >= 0; --d) { full[d] = (unsigned)(rem % ss[d]); rem /= ss[d]; }
-    bool ok = true;
-    for (int d = 0; d < nd; d++)
-      if (a.rs[d] == 1 && full[d] != 0) ok = false;
-    if (!ok) continue;
-    Term t;
-    t.idx = lin;
-    for (int e = 0; e < ne; e++) t.m.push_back(full[eff[e]]);
-    terms.push_back(t);
-  }
-  if (terms.empty()) return false;
-  // ascending X index: ascending m if the small operand is X, descending if it is Y (as launch_mul_stencil)
-  std::sort(terms.begin(), terms.end(), [&](const Term& x, const Term& y) { return small_is_x ? x.m < y.m : x.m > y.m; });
-  p.nt = (int)terms.size();
-  for (int t = 0; t < p.nt; t++) {
-    for (int e = 0; e < ne; e++) p.m[t][e] = (unsigned char)terms[t].m[e];
-    p.sidx[t] = (unsigned short)terms[t].idx;
-    bool new_group = t == 0;
-    for (int e = 0; e < ne - 1 && !new_group; e++) new_group = terms[t].m[e] != terms[t - 1].m[e];
-    p.group_start[t] = new_group ? 1 : 0;
-  }
+  set_terms(&p, small_terms(ss, eff, ne, !small_is_x));   // ascending X index
   p.self = small_is_x ? a.y : a.x;    // unused (no Add), any valid pointer
   p.subst = small_is_x ? a.x : a.y;
   p.res0 = small_is_x ? a.y : a.x;
@@ -1112,8 +1047,11 @@ bool launch_stencil_rows(Ctx& ctx, const MulArgs& a) {
   p.i_top = 0;
   p.nsteps = 1;
   p.bar = nullptr;   // a single step never reaches the grid barrier
-  if (ctx.direct_products && launch_direct_variant(ctx, p, 0, fs, total, "k_horner_direct<product>")) return true;
-  return ctx.bulk_products && launch_rows_variant(ctx, p, 0, fs, total, "k_horner_rows<product>");
+  HornerLaunch pl;
+  if ((ctx.direct_products && plan_direct_variant(ctx, p, 0, fs, total, "k_horner_direct<product>", &pl)) ||
+      (ctx.bulk_products && plan_rows_variant(ctx, p, 0, fs, total, "k_horner_rows<product>", &pl)))
+    return std::make_shared<const HornerLaunch>(pl);
+  return nullptr;
 }
 
 }  // namespace gtp

@@ -222,33 +222,14 @@ bool blk_mul_applicable(const Ctx& ctx, const MulArgs& a);
 void launch_mul_blk(Ctx& ctx, const MulArgs& a);
 bool slide_mul_applicable(const Ctx& ctx, const MulArgs& a);
 void launch_mul_slide(Ctx& ctx, const MulArgs& a);
-bool launch_mul_axis(Ctx& ctx, const MulArgs& a);   // kernels_mul_axis.cu
-bool launch_stencil_rows(Ctx& ctx, const MulArgs& a);   // kernels_horner.cu: row-staged (bulk-copy) small-operand product
-
-// 0: reference-order kernel, 2: 2x2-blocked DFMA kernel (kernels_mul_blk.cu), 3: sliding 1x2 DFMA kernel for dense
-// cube slabs (kernels_mul_slide.cu).  (1 was the cube-16-only kernel of
-// the first round; the blocked kernel with folded tables superseded it.)
-static int pad_plan(const Ctx& ctx, const MulArgs& a, MulArgs* out_best);
-// what launch_mul() will run -- 0: reference-order family (reference-order kernel, small-operand stencil, axis convolution:
-// all bit-exact), 2 / 3: blocked / sliding DFMA kernel, 6 / 7: the same after zero-extending odd extents
-int mul_plan_kind(const Ctx& ctx, const MulArgs& a) {
-  const int k = mul_kernel_kind(ctx, a);
-  if (k || !ctx.fast_mul) return k;
-  if (ctx.use_stencil && std::min(prod(a.xs), prod(a.ys)) <= (u64)32 && std::max(prod(a.xs), prod(a.ys)) >= 4096) return 0;
-  int nonunit_x = 0, nonunit_y = 0;
-  for (int d = 0; d < a.ndim; d++) { nonunit_x += a.xs[d] > 1; nonunit_y += a.ys[d] > 1; }
-  if (ctx.use_axis && (nonunit_x == 1) != (nonunit_y == 1)) return 0;   // axis convolution (bit-exact)
-  MulArgs best;
-  const int pk = pad_plan(ctx, a, &best);
-  return pk ? pk + 4 : 0;
-}
-int mul_kernel_kind(const Ctx& ctx, const MulArgs& a) {
-  if (!ctx.fast_mul) return 0;
-  if ((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.y)) & 15u) return 0;  // cp.async 16-byte staging
-  if (ctx.use_stencil && std::min(prod(a.xs), prod(a.ys)) <= (u64)32 && std::max(prod(a.xs), prod(a.ys)) >= 4096) return 0;  // stencil kernel
-  if (ctx.use_slide && slide_mul_applicable(ctx, a)) return 3;
-  return blk_mul_applicable(ctx, a) ? 2 : 0;
-}
+// kernels_mul_axis.cu: the axis convolution (null: not applicable)
+struct AxisPlan;
+std::shared_ptr<const AxisPlan> plan_mul_axis(const Ctx& ctx, const MulArgs& a);
+void launch_mul_axis(Ctx& ctx, const AxisPlan& pl);
+// kernels_horner.cu: the small-operand product on a row-walking / row-staged Horner kernel (null: not applicable)
+struct HornerLaunch;
+std::shared_ptr<const HornerLaunch> plan_small_rows(const Ctx& ctx, const MulArgs& a);
+void launch_horner_plan(Ctx& ctx, const HornerLaunch& pl);
 
 static void launch_mul_ordered(Ctx& ctx, const MulArgs& a) {
   const int nd = a.ndim;
@@ -456,16 +437,66 @@ __global__ void __launch_bounds__(256) k_mul_stencil_v4(const __grid_constant__ 
   }
 }
 
-// Returns false if the product is not a stencil case (then the caller falls back to the reference-order kernel).
-static bool launch_mul_stencil(Ctx& ctx, const MulArgs& a) {
+SmallTerms small_terms(const Shape& ss, const int* eff, int ne, bool descending) {
+  SmallTerms st;
+  memset(&st, 0, sizeof(st));
+  const int nd = (int)ss.size(), ns = (int)prod(ss);
+  u64 str[MAXD];
+  for (int d = nd - 1, s = 1; d >= 0; s *= (int)ss[d], --d) str[d] = (u64)s;
+  unsigned char m[SMALL_MAXT][SMALL_MAXE] = {};
+  int order[SMALL_MAXT];
+  for (int lin = 0; lin < ns; lin++) {
+    for (int e = 0; e < ne; e++) m[lin][e] = (unsigned char)(lin / str[eff[e]] % ss[eff[e]]);
+    order[lin] = lin;
+  }
+  // the keys are distinct: the small operand has extent 1 off the effective axes
+  std::sort(order, order + ns, [&](int x, int y) {
+    return descending ? std::lexicographical_compare(m[y], m[y] + ne, m[x], m[x] + ne)
+                      : std::lexicographical_compare(m[x], m[x] + ne, m[y], m[y] + ne);
+  });
+  st.nt = ns;
+  for (int t = 0; t < ns; t++) {
+    memcpy(st.m[t], m[order[t]], ne);
+    st.sidx[t] = (unsigned short)order[t];
+    st.group_start[t] = t == 0 || memcmp(st.m[t], st.m[t - 1], ne - 1) != 0;
+  }
+  return st;
+}
+
+// The products of an operand of at most ST_MAXT coefficients with one of at least 4096: HBM-bound, so the small-operand
+// kernels' and never the DFMA kernels'.
+static bool small_operand_product(const MulArgs& a) {
+  const u64 nx = prod(a.xs), ny = prod(a.ys);
+  return std::min(nx, ny) <= (u64)ST_MAXT && std::max(nx, ny) >= 4096;
+}
+
+struct StencilPlan {
+  StencilP p;
+  int grid;
+  bool v4;   // k_mul_stencil_v4 (p.total counts units of four), else k_mul_stencil
+};
+
+// The product's route through launch_mul and what each route launches
+enum MulRoute { MR_ORDERED, MR_BLK, MR_SLIDE, MR_SMALL_ROWS, MR_STENCIL, MR_AXIS, MR_PADDED };
+struct MulPlan {
+  MulRoute route = MR_ORDERED;
+  int kind = 0;                                // mul_kernel_kind
+  MulArgs a;                                   // the product; a row list also sets row_begin / row_step / row_count
+  std::shared_ptr<const HornerLaunch> rows;    // MR_SMALL_ROWS
+  StencilPlan stencil;                         // MR_STENCIL
+  std::shared_ptr<const AxisPlan> axis;        // MR_AXIS
+  MulArgs padded;                              // MR_PADDED: the zero-extended product (kind 6: blocked, 7: sliding)
+};
+
+// Small-operand product (small_operand_product holds): the Horner kernels' plan, else the stencil kernels'.  false: neither.
+static bool plan_small(const Ctx& ctx, const MulArgs& a, MulPlan* pl) {
   const int nd = a.ndim;
   if (a.accumulate || !a.rows.empty() || nd == 0 || nd > MAXD) return false;
   const u64 nx = prod(a.xs), ny = prod(a.ys);
   const bool small_is_x = nx <= ny;
   const Shape& ss = small_is_x ? a.xs : a.ys;
   const Shape& bs = small_is_x ? a.ys : a.xs;
-  const u64 ns = std::min(nx, ny), nb = std::max(nx, ny);
-  if (ns == 0 || ns > (u64)ST_MAXT || nb < 4096) return false;
+  if (std::min(nx, ny) == 0) return false;
   u64 row_elems = 1;
   for (int i = 1; i < nd; i++) row_elems *= a.rs[i];
   const u64 row_count = a.rs[0] == 1 ? 1 : a.row_count;
@@ -473,18 +504,20 @@ static bool launch_mul_stencil(Ctx& ctx, const MulArgs& a) {
   if (total == 0 || total >= (1ull << 32) - 65536 || a.row_begin + a.row_count * a.row_step >= (1ull << 32)) return false;
   for (int d = 0; d < nd; d++)
     if (ss[d] > 255) return false;
-  // The row-staged bulk-copy kernel (kernels_horner.cu) wins inside the fused Horner loop (0.138 s against 0.202 s on
-  // population_50_3vars --limit 300) but not on a single product, where the four-coefficient gather below is 2x faster
-  // (0.139 ms against 0.269 ms on [297,282,297] x [2,1,2], profiles/r02_stencil_ab.txt): opt-in for A/B measurements.
-  if ((ctx.bulk_products || ctx.direct_products) && launch_stencil_rows(ctx, a)) return true;
-  StencilP p;
-  memset(&p, 0, sizeof(p));
-  Shape sst(nd, 1), bst(nd, 1);
-  for (int i = nd - 2; i >= 0; --i) {
-    sst[i] = sst[i + 1] * ss[i + 1];
-    bst[i] = bst[i + 1] * bs[i + 1];
+  // The row-walking kernel (k_horner_direct, kernels_horner.cu) runs the products whose last effective axis has at least
+  // 192 coefficients (Ctx::direct_products, on by default: 0.119 against 0.137 ms).  The row-staged bulk-copy kernel wins
+  // inside the fused Horner loop (0.138 s against 0.202 s on population_50_3vars --limit 300) but not on a single product,
+  // where the four-coefficient gather below is 2x faster (0.139 ms against 0.269 ms on [297,282,297] x [2,1,2],
+  // profiles/r02_stencil_ab.txt): Ctx::bulk_products is opt-in, for A/B measurements.
+  if ((ctx.bulk_products || ctx.direct_products) && (pl->rows = plan_small_rows(ctx, a))) {
+    pl->route = MR_SMALL_ROWS;
+    return true;
   }
-  std::vector<int> eff;   // effective (non-unit result) axes
+  StencilP& p = pl->stencil.p;
+  memset(&p, 0, sizeof(p));
+  Shape bst(nd, 1);
+  for (int i = nd - 2; i >= 0; --i) bst[i] = bst[i + 1] * bs[i + 1];
+  int eff[MUL_MAXE], ne = 0;   // effective (non-unit result) axes
   for (int d = 0; d < nd; d++) {
     if (a.rs[d] == 1) {
       if (d == 0 && !(a.row_count <= 1 && a.row_begin == 0)) return false;
@@ -493,10 +526,10 @@ static bool launch_mul_stencil(Ctx& ctx, const MulArgs& a) {
       if (a.xs[d] != 1 || a.ys[d] != 1) return false;
       continue;
     }
-    eff.push_back(d);
+    if (ne == MUL_MAXE) return false;
+    eff[ne++] = d;
   }
-  if (eff.empty() || (int)eff.size() > MUL_MAXE) return false;
-  const int ne = (int)eff.size();
+  if (ne == 0) return false;
   p.ne = ne;
   p.row_axis = eff[0] == 0 ? 1 : 0;
   for (int e = 0; e < ne; e++) {
@@ -504,72 +537,50 @@ static bool launch_mul_stencil(Ctx& ctx, const MulArgs& a) {
     p.big[e] = (unsigned)bs[eff[e]];
     p.bstr[e] = (long long)bst[eff[e]];
   }
-  // the small operand's coefficients that can contribute (index 0 on every unit result axis), in visiting order:
-  // ascending X index <=> ascending m if the small operand is X, descending m if it is Y
-  struct Term { std::vector<unsigned> m; u64 idx; };
-  std::vector<Term> terms;
-  for (u64 lin = 0; lin < ns; lin++) {
-    u64 rem = lin;
-    std::vector<unsigned> full(nd);
-    for (int d = nd - 1; d >= 0; --d) {
-      full[d] = (unsigned)(rem % ss[d]);
-      rem /= ss[d];
-    }
-    bool ok = true;
-    for (int d = 0; d < nd; d++)
-      if (a.rs[d] == 1 && full[d] != 0) ok = false;
-    if (!ok) continue;
-    Term t;
-    t.idx = lin;
-    for (int e = 0; e < ne; e++) t.m.push_back(full[eff[e]]);
-    terms.push_back(t);
-  }
-  if (terms.empty()) return false;
-  std::sort(terms.begin(), terms.end(), [&](const Term& x, const Term& y) { return small_is_x ? x.m < y.m : x.m > y.m; });
-  p.nt = (int)terms.size();
-  for (int t = 0; t < p.nt; t++) {
-    long long delta = 0;
-    for (int e = 0; e < ne; e++) {
-      p.m[t][e] = (unsigned char)terms[t].m[e];
-      delta += (long long)terms[t].m[e] * p.bstr[e];
-    }
-    p.delta[t] = delta;
-    p.sidx[t] = (unsigned short)terms[t].idx;
-    bool new_group = t == 0;
-    for (int e = 0; e < ne - 1 && !new_group; e++) new_group = terms[t].m[e] != terms[t - 1].m[e];
-    p.group_start[t] = new_group ? 1 : 0;
-  }
+  const SmallTerms st = small_terms(ss, eff, ne, !small_is_x);
+  static_assert(sizeof(p.m) == sizeof(st.m), "StencilP holds the term table as it is built");
+  p.nt = st.nt;
+  memcpy(p.m, st.m, sizeof(p.m));
+  memcpy(p.sidx, st.sidx, sizeof(p.sidx));
+  memcpy(p.group_start, st.group_start, sizeof(p.group_start));
+  for (int t = 0; t < p.nt; t++)
+    for (int e = 0; e < ne; e++) p.delta[t] += (long long)p.m[t][e] * p.bstr[e];
   p.row_begin = (unsigned)a.row_begin;
   p.row_step = (unsigned)a.row_step;
   p.total = (unsigned)total;
   p.bigp = small_is_x ? a.y : a.x;
   p.smallp = small_is_x ? a.x : a.y;
   p.out = a.out;
-  const int block = 256;
-  const int grid = (int)std::max<u64>(1, std::min<u64>((total + block - 1) / block, (u64)ctx.sm_count * 32));
-  const int bucket = p.nt <= 2 ? 2 : p.nt <= 4 ? 4 : p.nt <= 8 ? 8 : p.nt <= 16 ? 16 : 32;
-  if (ne >= 2 && p.rs[ne - 1] >= 8 && p.bstr[ne - 1] == 1 && ctx.stencil_v4) {
+  pl->stencil.v4 = ne >= 2 && p.rs[ne - 1] >= 8 && p.bstr[ne - 1] == 1 && ctx.stencil_v4;
+  if (pl->stencil.v4) {
     p.lastq = (p.rs[ne - 1] + 3) / 4;
-    const u64 units = (total / p.rs[ne - 1]) * p.lastq;
-    p.total = (unsigned)units;
-    const int gridv = (int)std::max<u64>(1, std::min<u64>((units + block - 1) / block, (u64)ctx.sm_count * 32));
-#define CASE_NT(N, T) case T: GTP_LAUNCH(ctx, (k_mul_stencil_v4<N, T>), gridv, block, 0, p); break;
+    p.total = (unsigned)((total / p.rs[ne - 1]) * p.lastq);
+  }
+  pl->stencil.grid = (int)std::max<u64>(1, std::min<u64>((p.total + 255) / 256, (u64)ctx.sm_count * 32));
+  pl->route = MR_STENCIL;
+  return true;
+}
+
+static void launch_stencil(Ctx& ctx, const StencilPlan& pl) {
+  const StencilP& p = pl.p;
+  const int bucket = p.nt <= 2 ? 2 : p.nt <= 4 ? 4 : p.nt <= 8 ? 8 : p.nt <= 16 ? 16 : 32;
+  if (pl.v4) {
+#define CASE_NT(N, T) case T: GTP_LAUNCH(ctx, (k_mul_stencil_v4<N, T>), pl.grid, 256, 0, p); break;
 #define CASE(N) case N: switch (bucket) { CASE_NT(N, 2) CASE_NT(N, 4) CASE_NT(N, 8) CASE_NT(N, 16) CASE_NT(N, 32) } break;
-    switch (ne) {
+    switch (p.ne) {
       CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8)
     }
 #undef CASE
 #undef CASE_NT
-    return true;
+    return;
   }
-#define CASE_NT(N, T) case T: GTP_LAUNCH(ctx, (k_mul_stencil<N, T>), grid, block, 0, p); break;
+#define CASE_NT(N, T) case T: GTP_LAUNCH(ctx, (k_mul_stencil<N, T>), pl.grid, 256, 0, p); break;
 #define CASE(N) case N: switch (bucket) { CASE_NT(N, 2) CASE_NT(N, 4) CASE_NT(N, 8) CASE_NT(N, 16) CASE_NT(N, 32) } break;
-  switch (ne) {
+  switch (p.ne) {
     CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8)
   }
 #undef CASE
 #undef CASE_NT
-  return true;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -585,12 +596,13 @@ static u64 pad_chunkable(u64 l) {
   for (u64 c = l;; c++)
     if (dfma_chunk(c)) return c;
 }
-// 0: no padded plan; 2 / 3: zero-extend and run the blocked / sliding kernel on `best`
-static int pad_plan(const Ctx& ctx, const MulArgs& a, MulArgs* out_best) {
+
+// Zero-extension onto the sliding kernel (kind 7) or the blocked one (kind 6).  false: neither.
+static bool plan_padded(const Ctx& ctx, const MulArgs& a, MulPlan* pl) {
   const int nd = a.ndim;
-  if (nd < 3 || a.accumulate || !ctx.use_pad) return 0;
+  if (nd < 3 || a.accumulate || !ctx.use_pad) return false;
   const double macs = args_macs(a);
-  if (macs < 4.0 * DFMA_MIN_MACS) return 0;
+  if (macs < 4.0 * DFMA_MIN_MACS) return false;
   auto padded = [&](bool slide) {
     MulArgs m = a;
     m.rs[nd - 1] = pad_chunkable(a.rs[nd - 1]);
@@ -609,23 +621,24 @@ static int pad_plan(const Ctx& ctx, const MulArgs& a, MulArgs* out_best) {
     MulArgs m = padded(true);
     // (the sliding kernel runs ~1.4x faster per MAC than the blocked one: it wins up to ~2x padded work against the
     // blocked kernel's last-axis-only padding -- 5 x 17: planes 18, rows 20, last axis 20 = 1.99x the MACs)
-    if (slide_mul_applicable(ctx, m) && args_macs(m) <= 2.05 * macs) { best = m; kind = 3; }
+    if (slide_mul_applicable(ctx, m) && args_macs(m) <= 2.05 * macs) { best = m; kind = 7; }
   }
   if (!kind) {
     MulArgs m = padded(false);
-    if (blk_mul_applicable(ctx, m) && args_macs(m) <= 2.5 * macs) { best = m; kind = 2; }
+    if (blk_mul_applicable(ctx, m) && args_macs(m) <= 2.5 * macs) { best = m; kind = 6; }
   }
-  if (kind) *out_best = best;
-  return kind;
-}
-static bool launch_mul_padded(Ctx& ctx, const MulArgs& a) {
-  const int nd = a.ndim;
-  MulArgs best;
-  const int kind = pad_plan(ctx, a, &best);
   if (!kind) return false;
   auto tail_elems = [&](const Shape& s) { u64 p = 1; for (int d = 1; d < nd; d++) p *= s[d]; return p; };
   const u64 rows = a.rows.empty() ? a.row_count : a.rows.size();
   if (prod(best.xs) >= (1ull << 32) - 4096 || prod(best.ys) >= (1ull << 32) - 4096 || rows * tail_elems(best.rs) >= (1ull << 32) - 4096) return false;
+  pl->route = MR_PADDED;
+  pl->kind = kind;
+  pl->padded = best;
+  return true;
+}
+
+static void launch_mul_padded(Ctx& ctx, const MulArgs& a, MulArgs best, bool slide) {
+  const u64 rows = a.rows.empty() ? a.row_count : a.rows.size();
   auto pad_operand = [&](const double* src, const Shape& from, const Shape& to) -> BufP {
     if (from == to) return BufP();
     BufP b = ctx.alloc(prod(to));
@@ -644,47 +657,20 @@ static bool launch_mul_padded(Ctx& ctx, const MulArgs& a) {
   best.x = xp ? xp->d : a.x;
   best.y = yp ? yp->d : a.y;
   best.out = zp->d;
-  if (kind == 3) launch_mul_slide(ctx, best);
+  if (slide) launch_mul_slide(ctx, best);
   else launch_mul_blk(ctx, best);
   EwOperand Z;   // crop: the leading box of the padded rows
   Z.p = zp->d;
   Z.shape = zrows_p;
   launch_ew(ctx, EW_COPY, zrows, Z, nullptr, a.out, zrows, {});
-  return true;
 }
 
-void launch_mul(Ctx& ctx, const MulArgs& a_in) {
-  MulArgs a = a_in;
-  if (!a.rows.empty()) {
-    a.row_count = a.rows.size();
-    a.row_begin = a.rows[0];
-    a.row_step = 1;
-  }
-  const int kind = mul_kernel_kind(ctx, a);
-  if (ctx.hist) {   // GTP_LAUNCH_HIST=1: log every product above 10^6 MACs (shape census of real programs)
-    const double macs = args_macs(a);
-    if (macs >= 1e6) {
-      auto sh = [](const Shape& v) { std::string t; for (u64 x : v) t += std::to_string(x) + ","; return t; };
-      fprintf(stderr, "[gtp mul] kind %d macs %.3g x [%s] y [%s] r [%s] rows %llu\n", kind, macs, sh(a.xs).c_str(), sh(a.ys).c_str(),
-              sh(a.rs).c_str(), (unsigned long long)a.row_count);
-    }
-  }
-  if (kind == 2) {
-    launch_mul_blk(ctx, a);
-    return;
-  }
-  if (kind == 3) {
-    launch_mul_slide(ctx, a);
-    return;
-  }
-  if (ctx.fast_mul && ctx.use_stencil && launch_mul_stencil(ctx, a)) return;   // bit-exact, HBM-bound small-operand products
-  if (ctx.fast_mul && ctx.use_axis && launch_mul_axis(ctx, a)) return;         // bit-exact, 1-d operand x N-d tensor
-  if (ctx.fast_mul && launch_mul_padded(ctx, a)) return;                       // odd extents: zero-extend, DFMA kernels, crop
+// The reference-order kernel walks arithmetic progressions: one launch per maximal run of a row list
+static void launch_mul_reference(Ctx& ctx, const MulArgs& a) {
   if (a.rows.empty()) {
     launch_mul_ordered(ctx, a);
     return;
   }
-  // the reference-order kernel walks arithmetic progressions: one launch per maximal run of the list
   u64 row_elems = 1;
   for (int i = 1; i < a.ndim; i++) row_elems *= a.rs[i];
   size_t i = 0;
@@ -704,6 +690,67 @@ void launch_mul(Ctx& ctx, const MulArgs& a_in) {
     seg.out = a.out + i * row_elems;
     launch_mul_ordered(ctx, seg);
     i = j;
+  }
+}
+
+// Routes in order: the DFMA kernels (sliding, blocked), the small-operand kernels (bit-exact, HBM-bound), the axis
+// convolution (bit-exact, 1-d operand x N-d tensor), zero-extension onto the DFMA kernels (odd extents), and the
+// reference-order kernel.  Host only: nothing is launched.
+static MulPlan plan_mul(const Ctx& ctx, const MulArgs& a_in) {
+  MulPlan pl;
+  pl.a = a_in;
+  MulArgs& a = pl.a;
+  if (!a.rows.empty()) {
+    a.row_count = a.rows.size();
+    a.row_begin = a.rows[0];
+    a.row_step = 1;
+  }
+  if (!ctx.fast_mul) return pl;
+  const bool small = ctx.use_stencil && small_operand_product(a);
+  const bool aligned = !((reinterpret_cast<uintptr_t>(a.x) | reinterpret_cast<uintptr_t>(a.y)) & 15u);   // cp.async 16-byte staging
+  if (aligned && !small) {
+    if (ctx.use_slide && slide_mul_applicable(ctx, a)) {
+      pl.route = MR_SLIDE;
+      pl.kind = 3;
+      return pl;
+    }
+    if (blk_mul_applicable(ctx, a)) {
+      pl.route = MR_BLK;
+      pl.kind = 2;
+      return pl;
+    }
+  }
+  if (small && plan_small(ctx, a, &pl)) return pl;
+  if (ctx.use_axis && (pl.axis = plan_mul_axis(ctx, a))) {
+    pl.route = MR_AXIS;
+    return pl;
+  }
+  plan_padded(ctx, a, &pl);
+  return pl;
+}
+
+int mul_kernel_kind(const Ctx& ctx, const MulArgs& a) { return plan_mul(ctx, a).kind; }
+
+void launch_mul(Ctx& ctx, const MulArgs& a_in) {
+  const MulPlan pl = plan_mul(ctx, a_in);
+  const MulArgs& a = pl.a;
+  if (ctx.hist) {   // GTP_LAUNCH_HIST=1: log every product above 10^6 MACs (shape census of real programs)
+    const double macs = args_macs(a);
+    if (macs >= 1e6) {
+      const int kind = pl.route == MR_BLK || pl.route == MR_SLIDE ? pl.kind : 0;   // the DFMA kernel run on the operands as given
+      auto sh = [](const Shape& v) { std::string t; for (u64 x : v) t += std::to_string(x) + ","; return t; };
+      fprintf(stderr, "[gtp mul] kind %d macs %.3g x [%s] y [%s] r [%s] rows %llu\n", kind, macs, sh(a.xs).c_str(), sh(a.ys).c_str(),
+              sh(a.rs).c_str(), (unsigned long long)a.row_count);
+    }
+  }
+  switch (pl.route) {
+    case MR_BLK: launch_mul_blk(ctx, a); break;
+    case MR_SLIDE: launch_mul_slide(ctx, a); break;
+    case MR_SMALL_ROWS: launch_horner_plan(ctx, *pl.rows); break;
+    case MR_STENCIL: launch_stencil(ctx, pl.stencil); break;
+    case MR_AXIS: launch_mul_axis(ctx, *pl.axis); break;
+    case MR_PADDED: launch_mul_padded(ctx, a, pl.padded, pl.kind == 7); break;
+    case MR_ORDERED: launch_mul_reference(ctx, a); break;
   }
 }
 

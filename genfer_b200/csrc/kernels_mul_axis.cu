@@ -116,10 +116,18 @@ __global__ void __launch_bounds__(AX_TB) k_mul_axis_row(const AxisP p) {
   p.out[(size_t)o * p.Lr + k] = __dadd_rn(0.0, inner);
 }
 
-// Returns false when the product is not of this form (the caller goes on to the reference-order kernel).
-bool launch_mul_axis(Ctx& ctx, const MulArgs& a) {
+// The batched convolution's kernel and geometry (plan_mul_axis); launch_mul_axis launches exactly this
+struct AxisPlan {
+  AxisP p;
+  int KT;        // k_mul_axis_cols<KT>; 0: k_mul_axis_row
+  dim3 grid;
+  size_t smem;
+};
+
+// Null when the product is not of this form (the caller goes on to the next route).
+std::shared_ptr<const AxisPlan> plan_mul_axis(const Ctx& ctx, const MulArgs& a) {
   const int nd = a.ndim;
-  if (nd < 1 || a.accumulate || !a.rows.empty() || a.row_begin != 0 || a.row_step != 1 || a.row_count != a.rs[0]) return false;
+  if (nd < 1 || a.accumulate || !a.rows.empty() || a.row_begin != 0 || a.row_step != 1 || a.row_count != a.rs[0]) return nullptr;
   auto one_axis = [&](const Shape& s, int* ax) {
     int n = 0;
     for (int d = 0; d < nd; d++)
@@ -129,24 +137,25 @@ bool launch_mul_axis(Ctx& ctx, const MulArgs& a) {
   int ax = -1, ax2 = -1;
   const bool x1 = one_axis(a.xs, &ax), y1 = one_axis(a.ys, &ax2);
   bool small_is_x;
-  if (x1 && y1) return false;                       // 1-d times 1-d: tiny or the reference-order kernel's business
+  if (x1 && y1) return nullptr;                     // 1-d times 1-d: tiny or the reference-order kernel's business
   if (x1) small_is_x = true;
   else if (y1) { small_is_x = false; ax = ax2; }
-  else return false;
+  else return nullptr;
   const Shape& ss = small_is_x ? a.xs : a.ys;
   const Shape& bs = small_is_x ? a.ys : a.xs;
   for (int d = 0; d < nd; d++) {
-    if (d != ax && a.rs[d] != bs[d]) return false;  // the result keeps the big operand's extents off the axis (sum_shape)
-    if (bs[d] == 0 || a.rs[d] == 0) return false;
+    if (d != ax && a.rs[d] != bs[d]) return nullptr;  // the result keeps the big operand's extents off the axis (sum_shape)
+    if (bs[d] == 0 || a.rs[d] == 0) return nullptr;
   }
   const u64 Ls = ss[ax], Lb = bs[ax], Lr = a.rs[ax];
-  if (Ls < 2 || Lr > Lb + Ls - 1) return false;
+  if (Ls < 2 || Lr > Lb + Ls - 1) return nullptr;
   u64 outer = 1, inner = 1;
   for (int d = 0; d < ax; d++) outer *= bs[d];
   for (int d = ax + 1; d < nd; d++) inner *= bs[d];
-  if (outer * inner * std::max(Lb, Lr) >= (1ull << 31) || Ls >= (1u << 20)) return false;
-  if ((double)outer * inner * Lr * std::min(Ls, Lb) < 16384.0) return false;   // launch-bound either way
-  AxisP p;
+  if (outer * inner * std::max(Lb, Lr) >= (1ull << 31) || Ls >= (1u << 20)) return nullptr;
+  if ((double)outer * inner * Lr * std::min(Ls, Lb) < 16384.0) return nullptr;   // launch-bound either way
+  auto pl = std::make_shared<AxisPlan>();
+  AxisP& p = pl->p;
   p.big = small_is_x ? a.y : a.x;
   p.small = small_is_x ? a.x : a.y;
   p.out = a.out;
@@ -157,12 +166,11 @@ bool launch_mul_axis(Ctx& ctx, const MulArgs& a) {
   p.Lr = (unsigned)Lr;
   p.desc = small_is_x ? 0 : 1;   // ascending X index == descending index of a small Y
   if (inner == 1) {
-    const size_t smem = (2 * Ls + AX_TB) * sizeof(double);
-    if (smem > 200 * 1024 || outer > 65535) return false;
-    allow_dyn_smem(k_mul_axis_row, ctx.device, std::max<size_t>(smem, 48 * 1024));
-    dim3 grid((unsigned)((Lr + AX_TB - 1) / AX_TB), (unsigned)outer);
-    GTP_LAUNCH(ctx, k_mul_axis_row, grid, AX_TB, smem, p);
-    return true;
+    pl->smem = (2 * Ls + AX_TB) * sizeof(double);
+    if (pl->smem > 200 * 1024 || outer > 65535) return nullptr;
+    pl->KT = 0;
+    pl->grid = dim3((unsigned)((Lr + AX_TB - 1) / AX_TB), (unsigned)outer);
+    return pl;
   }
   // outputs per thread along the axis: 8 when that still gives every SM a few hundred threads, fewer for small tensors
   // ([336] x [336, 336]: KT = 8 left 14 k threads, each a chain of 336 dependent steps: 95 us; latency-bound)
@@ -170,15 +178,24 @@ bool launch_mul_axis(Ctx& ctx, const MulArgs& a) {
   int KT = 8;
   while (KT > 1 && ncol * ((Lr + KT - 1) / KT) < (u64)ctx.sm_count * 512) KT /= 2;
   const u64 ktiles = (Lr + KT - 1) / KT;
-  if (ktiles > 65535) return false;
-  dim3 grid((unsigned)((ncol + 127) / 128), (unsigned)ktiles);
-  switch (KT) {
-    case 8: GTP_LAUNCH(ctx, k_mul_axis_cols<8>, grid, 128, 0, p); break;
-    case 4: GTP_LAUNCH(ctx, k_mul_axis_cols<4>, grid, 128, 0, p); break;
-    case 2: GTP_LAUNCH(ctx, k_mul_axis_cols<2>, grid, 128, 0, p); break;
-    default: GTP_LAUNCH(ctx, k_mul_axis_cols<1>, grid, 128, 0, p); break;
+  if (ktiles > 65535) return nullptr;
+  pl->KT = KT;
+  pl->grid = dim3((unsigned)((ncol + 127) / 128), (unsigned)ktiles);
+  pl->smem = 0;
+  return pl;
+}
+
+void launch_mul_axis(Ctx& ctx, const AxisPlan& pl) {
+  switch (pl.KT) {
+    case 0:
+      allow_dyn_smem(k_mul_axis_row, ctx.device, std::max<size_t>(pl.smem, 48 * 1024));
+      GTP_LAUNCH(ctx, k_mul_axis_row, pl.grid, AX_TB, pl.smem, pl.p);
+      break;
+    case 8: GTP_LAUNCH(ctx, k_mul_axis_cols<8>, pl.grid, 128, 0, pl.p); break;
+    case 4: GTP_LAUNCH(ctx, k_mul_axis_cols<4>, pl.grid, 128, 0, pl.p); break;
+    case 2: GTP_LAUNCH(ctx, k_mul_axis_cols<2>, pl.grid, 128, 0, pl.p); break;
+    default: GTP_LAUNCH(ctx, k_mul_axis_cols<1>, pl.grid, 128, 0, pl.p); break;
   }
-  return true;
 }
 
 }  // namespace gtp

@@ -655,29 +655,11 @@ static std::shared_ptr<WaveTables> wave_tables(Ctx& ctx, const std::vector<u64>&
 
 template <int OP, bool EXACT>
 static bool wave_launch(Ctx& ctx, WaveP& p, unsigned want_ctas, size_t smem) {
-  static int coop[64] = {};           // 0 unknown, 1 yes, -1 no
-  int& c = coop[ctx.device & 63];
-  if (c == 0) {
-    int v = 0;
-    cudaDeviceGetAttribute(&v, cudaDevAttrCooperativeLaunch, ctx.device);
-    c = v ? 1 : -1;
-  }
-  if (c < 0) return false;
-  auto* fn = k_rec_wave<OP, EXACT>;
-  allow_dyn_smem(fn, ctx.device, smem);   // static + dynamic may pass 48 KB
-  int per_sm = 0;
-  GTP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, WV_T, smem));
-  if (per_sm < 1) return false;
+  const void* fn = (const void*)k_rec_wave<OP, EXACT>;
+  if (coop_ctas_per_sm(fn, ctx.device, WV_T, smem) == 0) return false;   // raises the smem limit: static + dynamic may pass 48 KB
   const unsigned max_ctas = (unsigned)ctx.sm_count;
   const unsigned grid = std::max(1u, std::min(want_ctas, max_ctas));
-  void* args[] = {(void*)&p};
-  const double t0 = ctx.hist ? Ctx::now() : 0.0;
-  GTP_CUDA(cudaLaunchCooperativeKernel((const void*)fn, dim3(grid), dim3(WV_T), args, smem, ctx.stream));
-  ctx.launches++;
-  if (ctx.hist) {
-    (*ctx.hist)[EXACT ? "k_rec_wave<exact>" : "k_rec_wave"]++;
-    ctx.t_launch += Ctx::now() - t0;
-  }
+  coop_launch(ctx, fn, grid, WV_T, smem, &p, EXACT ? "k_rec_wave<exact>" : "k_rec_wave");
   return true;
 }
 
