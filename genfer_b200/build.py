@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgenfer_taylor.so")
-SOURCES = ["api.cu", "api_uni.cu", "group.cu", "eval_api.cpp", "kernels_elem.cu", "kernels_mul.cu", "kernels_mul_blk.cu", "kernels_mul_slide.cu", "kernels_mul_axis.cu", "kernels_rec.cu", "kernels_wave.cu", "kernels_horner.cu", "interval_api.cu",
+SOURCES = ["api.cu", "api_uni.cu", "group.cu", "eval_api.cpp", "kernels_elem.cu", "kernels_mul.cu", "kernels_mul_blk.cu", "kernels_mul_slide.cu", "kernels_mul_box.cu", "kernels_mul_axis.cu", "kernels_rec.cu", "kernels_wave.cu", "kernels_horner.cu", "interval_api.cu",
            "univariate.cu"]
 HEADERS = ["common.hpp", "kernels.cuh", "device_sync.cuh", "interval.cuh", os.path.join("..", "..", "include", "genfer_taylor.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

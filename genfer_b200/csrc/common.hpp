@@ -216,6 +216,7 @@ struct Ctx {
   int fast_mul = 1;  // 0: reference-order kernel only, 1: auto, 2: force the blocked kernel even on tiny products (tests)
   std::shared_ptr<void> blk_plans;   // per-context caches of DFMA product plans (kernels_mul_blk.cu, dfma_plan_slot)
   std::shared_ptr<void> slide_plans; // same for kernels_mul_slide.cu
+  std::shared_ptr<void> box_plans;   // same for kernels_mul_box.cu
   std::shared_ptr<void> wave_tables; // level tables of the device-resident recurrences (kernels_wave.cu)
   bool bulk_products = false;        // also run plain small-operand products on the row-staged kernel (A/B; slower than the gather kernel)
   bool use_direct = true;            // row-walking plain-load variant of the Horner step (k_horner_direct), tried before the bulk-copy one

@@ -37,7 +37,9 @@ using IvP = std::unique_ptr<gti_poly>;
 namespace {
 
 constexpr int IVD = GTP_MAX_NDIM;
-constexpr int IVE = 12;   // non-unit axes a product / recurrence kernel handles
+// Non-unit axes a product / recurrence kernel handles: the kernels keep their per-axis state in arrays of E entries; tensors
+// of up to IVE non-unit axes run on the E = IVE instantiation, wider ones on E = IVD (more local memory per thread).
+constexpr int IVE = 12;
 
 // ------------------------------------------------------------------------------------------------------------------
 // kernels
@@ -100,20 +102,22 @@ __global__ void __launch_bounds__(256) k_iv_ew(const IvEwP p) {
 }
 
 // general truncated product in the reference's nesting order (`mul` :984-1012): see k_mul_ordered
+template <int E>
 struct IvMulP {
   int ne;
-  unsigned xs[IVE], ys[IVE], rs[IVE];
-  long long xstr[IVE], ystr[IVE];
+  unsigned xs[E], ys[E], rs[E];
+  long long xstr[E], ystr[E];
   u64 total;
   const Iv* x;
   const Iv* y;
   Iv* out;
 };
-__global__ void __launch_bounds__(128) k_iv_mul(const IvMulP p) {
+template <int E>
+__global__ void __launch_bounds__(128) k_iv_mul(const IvMulP<E> p) {
   const u64 gstride = (u64)gridDim.x * blockDim.x;
   const int NE = p.ne;
   for (u64 lin = (u64)blockIdx.x * blockDim.x + threadIdx.x; lin < p.total; lin += gstride) {
-    unsigned k[IVE], lo[IVE], hi[IVE], j[IVE];
+    unsigned k[E], lo[E], hi[E], j[E];
     u64 rem = lin;
     bool empty = false;
     for (int d = NE - 1; d >= 0; --d) {
@@ -164,10 +168,11 @@ __global__ void __launch_bounds__(128) k_iv_mul(const IvMulP p) {
 
 // div / exp / log, one total-degree level per launch: every coefficient of the level is an explicit function of coefficients of
 // lower levels (the forward substitutions of kernels_wave.cu, per coefficient).  op 0: r = x / y;  1: exp(x);  2: log(x).
+template <int E>
 struct IvLevP {
   int op, ne;
-  unsigned rs[IVE], xs[IVE], ys[IVE];
-  long long rstr[IVE], xstr[IVE], ystr[IVE];
+  unsigned rs[E], xs[E], ys[E];
+  long long rstr[E], xstr[E], ystr[E];
   u64 outer_total;   // prod(rs[0 .. ne-2])
   const Iv* x;
   const Iv* y;
@@ -176,11 +181,12 @@ struct IvLevP {
   int has_seed;
   Iv seed;           // exp / log of the constant term from the host's libm when the host knows it
 };
-__device__ __forceinline__ void iv_level_body(const IvLevP& p, unsigned level, u64 first, u64 gstride) {
+template <int E>
+__device__ __forceinline__ void iv_level_body(const IvLevP<E>& p, unsigned level, u64 first, u64 gstride) {
   const int ne = p.ne;
   const Iv zero = gti::iv(0.0, 0.0);
   for (u64 lin = first; lin < p.outer_total; lin += gstride) {
-    unsigned k[IVE];
+    unsigned k[E];
     u64 rem = lin;
     unsigned sum = 0;
     for (int d = ne - 2; d >= 0; --d) {
@@ -205,7 +211,7 @@ __device__ __forceinline__ void iv_level_body(const IvLevP& p, unsigned level, u
       else p.r[0] = p.has_seed ? p.seed : (p.op == 1 ? gti::iv_exp(p.x[0]) : gti::iv_log(p.x[0]));
       continue;
     }
-    unsigned lo[IVE], hi[IVE], m[IVE];   // inclusive bounds of the summation index
+    unsigned lo[E], hi[E], m[E];   // inclusive bounds of the summation index
     if (p.op == 0) {
       // r[k] = ((-sum_{m <= k, m != k, k - m < ys} r[m] * y[k - m]) + x[k]) / y[0]          (:1170-1191)
       bool any = true;
@@ -321,12 +327,14 @@ __device__ __forceinline__ void iv_level_body(const IvLevP& p, unsigned level, u
   }
 }
 
-__global__ void __launch_bounds__(128) k_iv_level(const IvLevP p, unsigned level) {
+template <int E>
+__global__ void __launch_bounds__(128) k_iv_level(const IvLevP<E> p, unsigned level) {
   iv_level_body(p, level, (u64)blockIdx.x * blockDim.x + threadIdx.x, (u64)gridDim.x * blockDim.x);
 }
 // Small tensors (1-d and thin 2-d series: hundreds of levels of a handful of coefficients each): ALL levels in one single-CTA
 // launch, a block barrier between levels (the level's coefficients are written and read by this CTA only).
-__global__ void __launch_bounds__(256) k_iv_levels_cta(const IvLevP p, unsigned levels) {
+template <int E>
+__global__ void __launch_bounds__(256) k_iv_levels_cta(const IvLevP<E> p, unsigned levels) {
   for (unsigned level = 0; level < levels; level++) {
     iv_level_body(p, level, threadIdx.x, blockDim.x);
     __syncthreads();
@@ -545,15 +553,15 @@ IvP poly_neg(Ctx& c, const gti_poly& a) {
   return r;
 }
 
-void launch_iv_mul(Ctx& c, const Iv* x, const Shape& xs, const Iv* y, const Shape& ys, Iv* out, const Shape& rs) {
+template <int E>
+void launch_iv_mul_e(Ctx& c, const Iv* x, const Shape& xs, const Iv* y, const Shape& ys, Iv* out, const Shape& rs) {
   const int nd = (int)rs.size();
-  IvMulP p;
+  IvMulP<E> p;
   memset(&p, 0, sizeof(p));
   Shape xst = strides_of(xs), yst = strides_of(ys);
   int ne = 0;
   for (int d = 0; d < nd; d++) {
     if (rs[d] == 1) continue;   // unit result axis: only index 0 of both operands contributes
-    GTP_CHECK(ne < IVE, GTP_ERR_ARG, "interval product: more than 12 non-unit result axes");
     p.xs[ne] = (unsigned)xs[d]; p.ys[ne] = (unsigned)ys[d]; p.rs[ne] = (unsigned)rs[d];
     p.xstr[ne] = (long long)xst[d]; p.ystr[ne] = (long long)yst[d];
     ne++;
@@ -568,7 +576,12 @@ void launch_iv_mul(Ctx& c, const Iv* x, const Shape& xs, const Iv* y, const Shap
   p.x = x; p.y = y; p.out = out;
   if (p.total == 0) return;
   const int grid = (int)std::max<u64>(1, std::min<u64>((p.total + 127) / 128, (u64)c.sm_count * 64));
-  GTP_LAUNCH(c, k_iv_mul, grid, 128, 0, p);
+  GTP_LAUNCH(c, k_iv_mul<E>, grid, 128, 0, p);
+}
+int nonunit_axes(const Shape& s) { return (int)std::count_if(s.begin(), s.end(), [](u64 x) { return x != 1; }); }
+void launch_iv_mul(Ctx& c, const Iv* x, const Shape& xs, const Iv* y, const Shape& ys, Iv* out, const Shape& rs) {
+  if (nonunit_axes(rs) <= IVE) launch_iv_mul_e<IVE>(c, x, xs, y, ys, out, rs);
+  else launch_iv_mul_e<IVD>(c, x, xs, y, ys, out, rs);
 }
 
 IvP poly_mul(Ctx& c, const gti_poly& a0, const gti_poly& b0) {   // :1014-1072
@@ -589,9 +602,10 @@ IvP poly_mul(Ctx& c, const gti_poly& a0, const gti_poly& b0) {   // :1014-1072
 }
 
 // div / exp / log by total-degree levels.  x, (y), r share ndim; r is dense over rs.
-void run_levels(Ctx& c, int op, const gti_poly& x, const gti_poly* y, gti_poly& r, const Iv* seed) {
+template <int E>
+void run_levels_e(Ctx& c, int op, const gti_poly& x, const gti_poly* y, gti_poly& r, const Iv* seed) {
   const int nd = (int)r.shape.size();
-  IvLevP p;
+  IvLevP<E> p;
   memset(&p, 0, sizeof(p));
   Shape xst = strides_of(x.shape), rst = strides_of(r.shape), yst;
   if (y) yst = strides_of(y->shape);
@@ -599,7 +613,6 @@ void run_levels(Ctx& c, int op, const gti_poly& x, const gti_poly* y, gti_poly& 
   u64 levels = 1;
   for (int d = 0; d < nd; d++) {
     if (r.shape[d] == 1) continue;
-    GTP_CHECK(ne < IVE, GTP_ERR_ARG, "interval recurrence: more than 12 non-unit result axes");
     p.rs[ne] = (unsigned)r.shape[d]; p.xs[ne] = (unsigned)x.shape[d]; p.ys[ne] = y ? (unsigned)y->shape[d] : 1u;
     p.rstr[ne] = (long long)rst[d]; p.xstr[ne] = (long long)xst[d]; p.ystr[ne] = y ? (long long)yst[d] : 0;
     levels += r.shape[d] - 1;
@@ -624,11 +637,15 @@ void run_levels(Ctx& c, int op, const gti_poly& x, const gti_poly* y, gti_poly& 
   p.has_seed = seed ? 1 : 0;
   if (seed) p.seed = *seed;
   if (p.outer_total <= 2048 && levels <= (1u << 20)) {
-    GTP_LAUNCH(c, k_iv_levels_cta, 1, 256, 0, p, (unsigned)levels);
+    GTP_LAUNCH(c, k_iv_levels_cta<E>, 1, 256, 0, p, (unsigned)levels);
     return;
   }
   const int grid = (int)std::max<u64>(1, std::min<u64>((p.outer_total + 127) / 128, (u64)c.sm_count * 32));
-  for (u64 t = 0; t < levels; t++) GTP_LAUNCH(c, k_iv_level, grid, 128, 0, p, (unsigned)t);
+  for (u64 t = 0; t < levels; t++) GTP_LAUNCH(c, k_iv_level<E>, grid, 128, 0, p, (unsigned)t);
+}
+void run_levels(Ctx& c, int op, const gti_poly& x, const gti_poly* y, gti_poly& r, const Iv* seed) {
+  if (nonunit_axes(r.shape) <= IVE) run_levels_e<IVE>(c, op, x, y, r, seed);
+  else run_levels_e<IVD>(c, op, x, y, r, seed);
 }
 
 IvP poly_div(Ctx& c, const gti_poly& a0, const gti_poly& b0) {   // :1194-1231

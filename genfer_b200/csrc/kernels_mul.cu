@@ -13,7 +13,7 @@
 
 namespace gtp {
 
-constexpr int MUL_MAXE = 8;  // effective (non-unit) result axes handled with register odometers
+constexpr int MUL_MAXE = 8;  // effective (non-unit) result axes of the small-operand kernels' parameter tables
 
 struct MulP {
   int ne;                       // effective axes
@@ -222,6 +222,9 @@ bool blk_mul_applicable(const Ctx& ctx, const MulArgs& a);
 void launch_mul_blk(Ctx& ctx, const MulArgs& a);
 bool slide_mul_applicable(const Ctx& ctx, const MulArgs& a);
 void launch_mul_slide(Ctx& ctx, const MulArgs& a);
+// kernels_mul_box.cu: the DFMA product for more than 8 effective axes
+bool box_mul_applicable(const Ctx& ctx, const MulArgs& a);
+void launch_mul_box(Ctx& ctx, const MulArgs& a);
 // kernels_mul_axis.cu: the axis convolution (null: not applicable)
 struct AxisPlan;
 std::shared_ptr<const AxisPlan> plan_mul_axis(const Ctx& ctx, const MulArgs& a);
@@ -251,7 +254,6 @@ static void launch_mul_ordered(Ctx& ctx, const MulArgs& a) {
       if (is_row) GTP_CHECK(a.row_count <= 1 && a.row_begin == 0, GTP_ERR_ARG, "row range on a unit leading axis");
       continue;  // unit result axis: only index 0 of both operands contributes
     }
-    GTP_CHECK(ne < MUL_MAXE, GTP_ERR_ARG, "more than 8 non-unit result axes are not supported yet");
     if (is_row) p.row_axis = 1;
     p.xs[ne] = (unsigned)a.xs[d];
     p.ys[ne] = (unsigned)a.ys[d];
@@ -281,9 +283,9 @@ static void launch_mul_ordered(Ctx& ctx, const MulArgs& a) {
     FusedClsArgs cls;
     if (fused_cls_begin(ctx, a.out, a.rs, &cls)) {
       const int blk = (int)std::min<u64>(1024, (p.total + 31) / 32 * 32);
-      switch (ne) {
+      switch (ne) {   // (1024 coefficients have at most 10 non-unit axes)
 #define CASE(N) case N: GTP_LAUNCH(ctx, k_mul_ordered_cls<N>, 1, blk, 0, p, cls); break;
-        CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8)
+        CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9) CASE(10)
 #undef CASE
       }
       return;
@@ -293,7 +295,8 @@ static void launch_mul_ordered(Ctx& ctx, const MulArgs& a) {
   int grid = (int)std::max<u64>(1, std::min<u64>((p.total + block - 1) / block, (u64)ctx.sm_count * 64));
   switch (ne) {
 #define CASE(N) case N: GTP_LAUNCH(ctx, k_mul_ordered<N>, grid, block, 0, p); break;
-    CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8)
+    CASE(1) CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9) CASE(10) CASE(11) CASE(12)
+    CASE(13) CASE(14) CASE(15) CASE(16) CASE(17) CASE(18) CASE(19) CASE(20) CASE(21) CASE(22) CASE(23) CASE(24)
 #undef CASE
   }
 }
@@ -477,7 +480,7 @@ struct StencilPlan {
 };
 
 // The product's route through launch_mul and what each route launches
-enum MulRoute { MR_ORDERED, MR_BLK, MR_SLIDE, MR_SMALL_ROWS, MR_STENCIL, MR_AXIS, MR_PADDED };
+enum MulRoute { MR_ORDERED, MR_BLK, MR_SLIDE, MR_SMALL_ROWS, MR_STENCIL, MR_AXIS, MR_PADDED, MR_BOX };
 struct MulPlan {
   MulRoute route = MR_ORDERED;
   int kind = 0;                                // mul_kernel_kind
@@ -694,8 +697,9 @@ static void launch_mul_reference(Ctx& ctx, const MulArgs& a) {
 }
 
 // Routes in order: the DFMA kernels (sliding, blocked), the small-operand kernels (bit-exact, HBM-bound), the axis
-// convolution (bit-exact, 1-d operand x N-d tensor), zero-extension onto the DFMA kernels (odd extents), and the
-// reference-order kernel.  Host only: nothing is launched.
+// convolution (bit-exact, 1-d operand x N-d tensor), zero-extension onto the DFMA kernels (odd extents), the trailing-box
+// DFMA kernel (more than 8 effective axes, from DFMA_MIN_MACS), and the reference-order kernel.  Host only: nothing is
+// launched.
 static MulPlan plan_mul(const Ctx& ctx, const MulArgs& a_in) {
   MulPlan pl;
   pl.a = a_in;
@@ -725,7 +729,11 @@ static MulPlan plan_mul(const Ctx& ctx, const MulArgs& a_in) {
     pl.route = MR_AXIS;
     return pl;
   }
-  plan_padded(ctx, a, &pl);
+  if (plan_padded(ctx, a, &pl)) return pl;
+  if (args_macs(a) >= DFMA_MIN_MACS && box_mul_applicable(ctx, a)) {
+    pl.route = MR_BOX;
+    pl.kind = 8;
+  }
   return pl;
 }
 
@@ -737,7 +745,7 @@ void launch_mul(Ctx& ctx, const MulArgs& a_in) {
   if (ctx.hist) {   // GTP_LAUNCH_HIST=1: log every product above 10^6 MACs (shape census of real programs)
     const double macs = args_macs(a);
     if (macs >= 1e6) {
-      const int kind = pl.route == MR_BLK || pl.route == MR_SLIDE ? pl.kind : 0;   // the DFMA kernel run on the operands as given
+      const int kind = pl.route == MR_BLK || pl.route == MR_SLIDE || pl.route == MR_BOX ? pl.kind : 0;   // the DFMA kernel run on the operands as given
       auto sh = [](const Shape& v) { std::string t; for (u64 x : v) t += std::to_string(x) + ","; return t; };
       fprintf(stderr, "[gtp mul] kind %d macs %.3g x [%s] y [%s] r [%s] rows %llu\n", kind, macs, sh(a.xs).c_str(), sh(a.ys).c_str(),
               sh(a.rs).c_str(), (unsigned long long)a.row_count);
@@ -750,6 +758,7 @@ void launch_mul(Ctx& ctx, const MulArgs& a_in) {
     case MR_STENCIL: launch_stencil(ctx, pl.stencil); break;
     case MR_AXIS: launch_mul_axis(ctx, *pl.axis); break;
     case MR_PADDED: launch_mul_padded(ctx, a, pl.padded, pl.kind == 7); break;
+    case MR_BOX: launch_mul_box(ctx, a); break;
     case MR_ORDERED: launch_mul_reference(ctx, a); break;
   }
 }
